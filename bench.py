@@ -50,6 +50,31 @@ def make_problems(count, first_seed):
     return [gen.homography(n=N_POINTS, inlier_ratio=INLIER_RATIO, seed=first_seed + i)[0] for i in range(count)]
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, fields):
+    """--dump-outputs: what the timed path returned for its last step, one DIR/<field>.npy per result field with one row per
+    fit, so that two builds can be compared output for output. float32 fields stay float32, integer fields are written as
+    float64 (exact below 2**53). Rows beyond 64 MB in all are sampled (fixed seed, ascending) and rows.npy names the kept ones."""
+    arrays = {k: np.asarray(v, np.float32 if np.asarray(v).dtype == np.float32 else np.float64) for k, v in fields.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values()) + 8
+    budget = DUMP_LIMIT - 256 * (len(arrays) + 1)          # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["rows"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def record_fields(rec):
+    """usac_fit_result records (GpuContext.fit_records) -> {field: array}."""
+    return {k: rec[k] for k in rec.dtype.names}
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # clocks sampler (NVML): SM clock + throttle reasons during the timed region
 # ---------------------------------------------------------------------------------------------------------------------
@@ -178,10 +203,12 @@ def run_reference_arm(args):
     evals = 0
     t = 0.0
     for _ in range(args.steps):
-        e, dt, _ = cpu_fits(problems, seeds, cores, impl)
+        e, dt, rs = cpu_fits(problems, seeds, cores, impl)
         evals += e
         t += dt
     v = evals / t
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: [r[k] for r in rs] for k in rs[0] if np.asarray(rs[0][k]).dtype.kind in "biuf"})
     sample = (f"{per_step} C2 image pairs per step, all host threads over independent fits; " +
               (REF_SAMPLE_NOTE if impl == "reference" else "CPU oracle (restated reference), oracle/libusac_oracle.so"))
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "evals/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -248,8 +275,10 @@ def run_native(args):
         barrier()
         return ev0.elapsed_time(ev1), stats
 
+    last = [None]          # the records of the latest resident step (--dump-outputs)
+
     def step_resident():
-        res = ctx.fit_records(**fit_kw)
+        res = last[0] = ctx.fit_records(**fit_kw)
         t = ctx.last_timing()
         return (int(res["useful_evals"].sum()), int(res["evals"].sum()), t["launches"], t["score_launches"], t["score_ms"],
                 int(res["iterations"].sum()), int(res["rounds"].max()), int(res["rounds"].sum()))
@@ -354,6 +383,7 @@ def run_native(args):
     ms, stats = timed(step_resident, args.steps)
     clk = clocks.stop()
     ms_single = ms
+    resident_out = last[0]
     for i, (lo_, hi_) in enumerate(halves):
         pipe_ctx[i].set_points(capi.EST_HOMOGRAPHY, host[lo_ * N_POINTS:hi_ * N_POINTS], sizes[lo_:hi_])
     timed_threads(step_resident_pipelined, args.warmup)
@@ -392,7 +422,7 @@ def run_native(args):
         for c2 in pipe_ctx + pipe_ctx2:
             c2.close()
         pipe_ctx, pipe_ctx2 = [], []
-        c5 = c5_leg(args, rank, world, local, max(5, args.steps), 3)
+        c5 = c5_leg(args, rank, world, local, args.steps, 3)
 
     h2d_all = torch.tensor([h2d_only_ms], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -465,11 +495,13 @@ def run_native(args):
         if c5 is not None:
             line["config"]["c5"] = c5
         if not args.no_epipolar:
-            line.update(epipolar_rooflines(local, fp32_peak, peak_source))
+            line.update(epipolar_rooflines(local, fp32_peak, peak_source, args.steps))
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_baseline()
         if args.latency:
             line["config"]["single_fit_latency_ms"] = single_fit_latency(ctx, problems[0], timed)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, record_fields(resident_out))
         print(json.dumps(line))
     ctx.close()
     for c2 in pipe_ctx + pipe_ctx2:
@@ -489,8 +521,9 @@ def run_native(args):
 C5_GOLDEN = os.path.join(ROOT, "tests", "golden", "c5_n1_oracle.json")   # the full 10 000-sample fit by the CPU oracle (committed)
 
 
-def c5_leg(args, rank, world, local, steps, warmup):
-    """-> dict for config.c5 (every rank returns it; identical on all ranks by construction and asserted so)."""
+def c5_leg(args, rank, world, local, steps, warmup, dump=None):
+    """-> dict for config.c5 (every rank returns it; identical on all ranks by construction and asserted so). `dump`: directory
+    for rank 0's fit record of the last timed step (--dump-outputs of --workload c5)."""
     import zlib
 
     import torch
@@ -525,8 +558,11 @@ def c5_leg(args, rank, world, local, steps, warmup):
         D.barrier(); torch.cuda.synchronize()
         return ev0.elapsed_time(ev1), out
 
+    last = [None]
+
     def step():
-        r = ctx.fit_records(**fit_kw)[0]
+        last[0] = ctx.fit_records(**fit_kw)
+        r = last[0][0]
         t = ctx.last_timing()
         return (int(r["useful_evals"]), int(r["evals"]), t["launches"], t["score_launches"], t["score_ms"], int(r["iterations"]), int(r["inliers"]),
                 int(r["best_hyp"]), zlib.crc32(np.asarray(r["model"], np.float32).tobytes()), int(r["rounds"]))
@@ -561,10 +597,11 @@ def c5_leg(args, rank, world, local, steps, warmup):
     clocks.start()
     ms, st = bracket(step, steps)
     clk = clocks.stop()
-    n_e2e = max(1, min(steps, 3))
-    ms_e2e, st_e2e = bracket(step_e2e, n_e2e)
-    t_all = D.reduce_max([ms / steps, ms_e2e / n_e2e])
-    sums = D.reduce_sum([sum(x[0] for x in st), sum(x[1] for x in st), sum(x[2] for x in st), sum(x[0] for x in st_e2e) / n_e2e])
+    if dump and rank == 0:
+        dump_outputs(dump, record_fields(last[0]))
+    ms_e2e, st_e2e = bracket(step_e2e, steps)
+    t_all = D.reduce_max([ms / steps, ms_e2e / steps])
+    sums = D.reduce_sum([sum(x[0] for x in st), sum(x[1] for x in st), sum(x[2] for x in st), sum(x[0] for x in st_e2e) / steps])
     # every rank must hold the same result (the gathered scores and select_kernel are identical everywhere)
     mine = [float(st[-1][5]), float(st[-1][6]), float(st[-1][7]), float(st[-1][8])]
     lo_, hi_ = D.reduce_max(mine), [-v for v in D.reduce_max([-v for v in mine])]
@@ -580,7 +617,7 @@ def c5_leg(args, rank, world, local, steps, warmup):
     peak = 2.0 * 128 * info["sm_count"] * info["sm_clock_khz"] * 1e3 / 1e12
     out = {"workload": f"C5 homography N={n}, 10% inliers (clustered), NAPSAC grid cell 50, max_iter {MAX_IT}, conf {CONF}; one robust fit, "
                        f"hypotheses of every round of {K} samples sharded over {world} GPU(s), one exchange of the per-sample scores per round",
-           "scaling": "strong", "exchange": exchange, "ms_per_fit_nccl": ms_nccl, "ms_per_fit": t_all[0], "evals_per_s": sums[0] / steps / (t_all[0] * 1e-3),
+           "scaling": "strong", "steps": steps, "exchange": exchange, "ms_per_fit_nccl": ms_nccl, "ms_per_fit": t_all[0], "evals_per_s": sums[0] / steps / (t_all[0] * 1e-3),
            "evals_executed_per_s": sums[1] / steps / (t_all[0] * 1e-3),
            "iterations": st[-1][5], "inliers": st[-1][6], "best_hyp": st[-1][7], "model_crc": st[-1][8], "rounds": st[-1][9],
            "parity_vs_n1": parity, "parity_note": "iterations / inliers / winning sample / model CRC32 equal tests/golden/c5_n1_oracle.json "
@@ -602,7 +639,7 @@ def run_c5(args):
         raise SystemExit("bench.py: no CUDA device - the product path has no CPU fallback")
     torch.cuda.set_device(local)
     rank, world = D.init("nccl")
-    c5 = c5_leg(args, rank, world, local, args.steps, max(args.warmup, 3))
+    c5 = c5_leg(args, rank, world, local, args.steps, max(args.warmup, 3), dump=args.dump_outputs)
     if rank == 0:
         line = {"metric": METRIC, "value": c5["evals_per_s"], "unit": "evals/s", "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
                 "ms_per_step": c5["ms_per_fit"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
@@ -642,7 +679,7 @@ def epipolar_rooflines(local, fp32_peak, peak_source, steps=6):
             ach = flops * ev / (best * 1e-3) / 1e12
             out[name] = {"bound": "fp32", "kernel": f"score_sq_kernel<{'FUNDAMENTAL' if est == capi.EST_FUNDAMENTAL else 'ESSENTIAL'}>", "achieved": ach,
                          "peak": fp32_peak, "unit": "TFLOP/s", "frac": ach / fp32_peak, "flops_per_eval": flops, "evals_per_launch": ev,
-                         "launch_ms": best, "peak_source": peak_source,
+                         "launch_ms": best, "steps": steps, "peak_source": peak_source,
                          "workload": f"{B} image pairs x {K} samples x {N_POINTS} correspondences, one scoring launch per fit"}
     return out
 
@@ -687,7 +724,13 @@ def main():
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"], help="c2: batch of independent N=4000 fits (default); c5: one 1M-point fit, hypotheses sharded")
     ap.add_argument("--c5-points", type=int, default=1000000)
     ap.add_argument("--c5-round", type=int, default=0, help="samples per round of the c5 leg (0 = 5000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the results of the last one (rank 0: one row per "
+                    "fit in image-pair order, every field of the fit record) as DIR/<field>.npy, float32 or float64, 64 MB at most. "
+                    "The GPU arms fit --problems pairs; the CPU arm (--impl reference) fits max(host cores, --ref-problems) pairs, "
+                    "so its dumps from hosts with other core counts agree on the common leading rows only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "native":
         args.warmup = max(args.warmup, 1)
     if args.impl == "reference":

@@ -11,6 +11,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "libusac_oracle.so")
+SHIM_LIB = os.path.join(_HERE, "libref_shim.so")      # the stand-in OpenCV numerics of ref_shim/ (ref_shim_entry.cpp), for oracle/ref.py
 
 EST_LINE2D, EST_HOMOGRAPHY, EST_FUNDAMENTAL, EST_ESSENTIAL = 1, 2, 3, 4
 SAMPLER_UNIFORM, SAMPLER_PROGRESSIVE_NAPSAC, SAMPLER_NAPSAC, SAMPLER_PROSAC = 1, 2, 3, 4
@@ -23,7 +24,8 @@ MAX_MODELS = {EST_LINE2D: 1, EST_HOMOGRAPHY: 1, EST_FUNDAMENTAL: 3, EST_ESSENTIA
 def build(force=False):
     """Compile the oracle with its Makefile (g++). Building the checker is not using it."""
     srcs = [os.path.join(_HERE, f) for f in os.listdir(_HERE) if f.endswith((".cpp", ".h"))]
-    if force or not os.path.exists(_LIB) or any(os.path.getmtime(s) > os.path.getmtime(_LIB) for s in srcs):
+    libs = (_LIB, SHIM_LIB)
+    if force or not all(os.path.exists(lib) for lib in libs) or any(os.path.getmtime(s) > os.path.getmtime(lib) for s in srcs for lib in libs):
         subprocess.check_call(["make", "-C", _HERE, "-s"])
     return _LIB
 

@@ -63,6 +63,19 @@ def lib():
     return _lib
 
 
+_shim = None
+
+
+def shim_lib():
+    """oracle/libref_shim.so: the stand-in OpenCV numerics alone (ref_shim_entry.cpp), built with the oracle - needs no reference."""
+    global _shim
+    if _shim is None:
+        from oracle import oracle as O
+        O.build()
+        _shim = C.CDLL(O.SHIM_LIB)
+    return _shim
+
+
 def _f(a):
     return a.ctypes.data_as(C.POINTER(C.c_float))
 
@@ -190,7 +203,7 @@ def shim_svd(A, depth64=False, flags=0):
     r, c = A.shape
     w, u, vt, dims = np.zeros(max(r, c)), np.zeros(max(r, c) ** 2), np.zeros(max(r, c) ** 2), np.zeros(5, np.int32)
     dp = C.POINTER(C.c_double)
-    fn = lib().ref_shim_svd
+    fn = shim_lib().ref_shim_svd
     fn.argtypes = [dp, C.c_int, C.c_int, C.c_int, C.c_int, dp, dp, dp, C.POINTER(C.c_int)]
     fn(A.ctypes.data_as(dp), r, c, int(depth64), int(flags), w.ctypes.data_as(dp), u.ctypes.data_as(dp), vt.ctypes.data_as(dp), _i(dims))
     return w[:dims[0]].copy(), u[:dims[1] * dims[2]].reshape(dims[1], dims[2]).copy(), vt[:dims[3] * dims[4]].reshape(dims[3], dims[4]).copy()
@@ -202,7 +215,7 @@ def shim_eigen(A, depth64=False):
     n = A.shape[0]
     ev, vec = np.zeros(n), np.zeros((n, n))
     dp = C.POINTER(C.c_double)
-    fn = lib().ref_shim_eigen
+    fn = shim_lib().ref_shim_eigen
     fn.argtypes = [dp, C.c_int, C.c_int, dp, dp]
     ok = fn(A.ctypes.data_as(dp), n, int(depth64), ev.ctypes.data_as(dp), vec.ctypes.data_as(dp))
     return (ev, vec) if ok else None
@@ -212,7 +225,7 @@ def shim_cubic(coeffs4):
     c = np.ascontiguousarray(coeffs4, dtype=np.float64)
     r = np.zeros(3)
     dp = C.POINTER(C.c_double)
-    fn = lib().ref_shim_cubic
+    fn = shim_lib().ref_shim_cubic
     fn.argtypes = [dp, dp]
     n = fn(c.ctypes.data_as(dp), r.ctypes.data_as(dp))
     return n, r
@@ -221,7 +234,7 @@ def shim_cubic(coeffs4):
 def shim_inv3(m):
     a = np.ascontiguousarray(m, dtype=np.float32).reshape(9)
     out = np.zeros(9, np.float32)
-    fn = lib().ref_shim_inv3
+    fn = shim_lib().ref_shim_inv3
     fn.argtypes = [C.POINTER(C.c_float), C.POINTER(C.c_float)]
     fn(_f(a), _f(out))
     return out.reshape(3, 3)
