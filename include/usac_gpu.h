@@ -29,6 +29,12 @@ enum { USAC_RNG_PHILOX = 1 /* counter based, keyed by (seed, hypothesis id) */,
 enum { USAC_OK = 0, USAC_ERR_CUDA = 1, USAC_ERR_ARG = 2, USAC_ERR_STATE = 3, USAC_ERR_NCCL = 4 };
 
 #define USAC_MAX_MODELS_PER_SAMPLE 3   /* seven-point cubic: up to 3 roots (ransac.cpp:24-28) */
+#define USAC_E5_MAX_ROOTS 10           /* five-point solver: up to 10 real roots, every cheirality-valid one a model (usac_fit_cfg::essential_roots) */
+/* usac_fit_cfg::essential_roots: which roots of a five-point sample become models */
+enum { USAC_E5_ROOTS_FIRST_VALID = 0 /* the reference's rule (default): the first root, in visiting order, that passes the
+                                        cheirality vote (five_points.cpp:217-262) */,
+       USAC_E5_ROOTS_ALL_VALID = 1   /* every root that passes it, up to USAC_E5_MAX_ROOTS, in visiting order; the fit treats
+                                        them as it treats the seven-point solver's roots (ransac.cpp:24-28) */ };
 
 typedef struct usac_gpu_ctx usac_gpu_ctx;
 
@@ -86,6 +92,9 @@ int usac_gpu_sample(usac_gpu_ctx* ctx, int problem, const usac_sampler_cfg* cfg,
 /* samples: K x m. models_out: K x S x 9 floats (S = 3 for fundamental, else 1; line models use the first 3 floats of
  * their 9-float slot), nmodels_out[K] = number of valid models of each sample (0 = degenerate). */
 int usac_gpu_estimate(usac_gpu_ctx* ctx, int problem, const int* samples, int K, float* models_out, int* nmodels_out);
+/* the five-point solver with USAC_E5_ROOTS_ALL_VALID (essential problems only): models_out K x USAC_E5_MAX_ROOTS x 9 floats, every
+ * cheirality-valid root of sample k in visiting order (ascending |z|), unused slots zero; nmodels_out[K] = how many (0..10) */
+int usac_gpu_estimate_essential_roots(usac_gpu_ctx* ctx, int problem, const int* samples, int K, float* models_out, int* nmodels_out);
 
 /* ---- fused robust fit: replaces the loop of Ransac::run (ransac.cpp:58-139) for every uploaded problem ---------- */
 typedef struct {
@@ -111,6 +120,9 @@ typedef struct {
     /* model.hpp:39: SPRT-rejected models of the first this-many hypotheses still get a full inlier count (sprt.hpp:243-257)
      * and do not burn an iteration (ransac.cpp:77-85). 0 = the reference default 20. */
     unsigned max_hypothesis_test_before_sprt;
+    /* USAC_E5_ROOTS_*: essential fits only (any other value, or a non-zero value for another estimator, is USAC_ERR_ARG).
+     * ALL_VALID needs fewer than 2^28 points per problem. 0 (a zero-initialised config) = the reference's rule. */
+    int essential_roots;
 } usac_fit_cfg;
 
 typedef struct {
@@ -120,7 +132,7 @@ typedef struct {
     unsigned iterations;         /* `iters` when the loop ended (RansacOutput::number_iterations) */
     unsigned samples_drawn;
     long long best_hyp;          /* sample id of the best model, -1 if none */
-    int best_model_idx;
+    int best_model_idx;          /* which model of that sample: 0..2 for fundamental, 0..9 for essential with USAC_E5_ROOTS_ALL_VALID, else 0 */
     unsigned rounds;
     unsigned long long evals;    /* hypothesis x point evaluations executed on this GPU (whole rounds) */
     unsigned long long useful_evals; /* the part of `evals` the sequential loop of ransac.cpp:58-139 would also have

@@ -9,8 +9,9 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .capi import (EST_ESSENTIAL, EST_FUNDAMENTAL, EST_HOMOGRAPHY, EST_LINE2D, MAX_MODELS, NEIGH_GRID, NEIGH_KNN,  # noqa: F401
-                   NEIGH_NONE, RNG_PHILOX, RNG_TABLE, SAMPLE_SIZE, SAMPLER_NAPSAC, SAMPLER_PROSAC, SAMPLER_UNIFORM)
+from .capi import (E5_MAX_ROOTS, E5_ROOTS_ALL_VALID, E5_ROOTS_FIRST_VALID, EST_ESSENTIAL, EST_FUNDAMENTAL,  # noqa: F401
+                   EST_HOMOGRAPHY, EST_LINE2D, MAX_MODELS, NEIGH_GRID, NEIGH_KNN, NEIGH_NONE, RNG_PHILOX, RNG_TABLE, SAMPLE_SIZE,
+                   SAMPLER_NAPSAC, SAMPLER_PROSAC, SAMPLER_UNIFORM)
 
 
 class UsacGpuError(RuntimeError):
@@ -137,12 +138,23 @@ class GpuContext:
         self._check(self.L.usac_gpu_estimate(self.h, problem, _ptr(s, C.c_int), K, _ptr(models, C.c_float), _ptr(nm, C.c_int)), "estimate")
         return models, nm
 
+    def estimate_essential_roots(self, samples, problem=0):
+        """Five-point solve keeping every cheirality-valid root -> (models [K, 10, 9], nmodels [K]); models in visiting order."""
+        s = np.ascontiguousarray(samples, dtype=np.int32).reshape(-1, SAMPLE_SIZE[EST_ESSENTIAL])
+        K = s.shape[0]
+        models = np.zeros((K, E5_MAX_ROOTS, 9), np.float32)
+        nm = np.zeros(K, np.int32)
+        self._check(self.L.usac_gpu_estimate_essential_roots(self.h, problem, _ptr(s, C.c_int), K, _ptr(models, C.c_float), _ptr(nm, C.c_int)),
+                    "estimate_essential_roots")
+        return models, nm
+
     # ---- fused fit ----
     def fit_records(self, threshold, confidence=0.95, max_iterations=10000, sampler=SAMPLER_UNIFORM, rng=RNG_PHILOX, seed=1,
                     sprt=False, round_size=0, neighbors=NEIGH_NONE, sample_table=None, rank=0, nranks=1, lo=0, lo_params=None,
-                    max_hypothesis_test_before_sprt=0):
+                    max_hypothesis_test_before_sprt=0, essential_roots=E5_ROOTS_FIRST_VALID):
         """One robust fit per uploaded problem; returns a numpy record array laid out as usac_fit_result (no per-problem
-        Python work: this is what a batched caller uses)."""
+        Python work: this is what a batched caller uses). essential_roots=E5_ROOTS_ALL_VALID (essential only): every
+        cheirality-valid five-point root is a model, so best_model_idx ranges over 0..9."""
         cfg = capi.FitCfg()
         cfg.sampler = capi.SamplerCfg(sampler, rng, seed, neighbors, 0, 0)
         cfg.threshold, cfg.confidence, cfg.max_iterations = threshold, confidence, max_iterations
@@ -150,6 +162,7 @@ class GpuContext:
         if lo_params is not None:     # (lo_sample_size, lo_inner_iterations, lo_iterative_iterations, lo_threshold_multiplier), model.hpp:26-29
             cfg.lo_sample_size, cfg.lo_inner_iterations, cfg.lo_iterative_iterations, cfg.lo_threshold_multiplier = [int(v) for v in lo_params]
         cfg.max_hypothesis_test_before_sprt = int(max_hypothesis_test_before_sprt)
+        cfg.essential_roots = int(essential_roots)
         if sample_table is not None:
             t = np.ascontiguousarray(sample_table, dtype=np.int32)
             self._table = t

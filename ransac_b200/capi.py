@@ -18,6 +18,8 @@ RNG_PHILOX, RNG_TABLE = 1, 2
 OK, ERR_CUDA, ERR_ARG, ERR_STATE, ERR_NCCL = 0, 1, 2, 3, 4
 SAMPLE_SIZE = {EST_LINE2D: 2, EST_HOMOGRAPHY: 4, EST_FUNDAMENTAL: 7, EST_ESSENTIAL: 5}
 MAX_MODELS = {EST_LINE2D: 1, EST_HOMOGRAPHY: 1, EST_FUNDAMENTAL: 3, EST_ESSENTIAL: 1}
+E5_MAX_ROOTS = 10
+E5_ROOTS_FIRST_VALID, E5_ROOTS_ALL_VALID = 0, 1
 
 
 class SamplerCfg(C.Structure):
@@ -30,7 +32,7 @@ class FitCfg(C.Structure):
                 ("sprt", C.c_int), ("round_size", C.c_int), ("sample_table", C.POINTER(C.c_int)),
                 ("sample_table_rows", C.c_uint), ("rank", C.c_int), ("nranks", C.c_int), ("lo", C.c_int),
                 ("lo_sample_size", C.c_uint), ("lo_inner_iterations", C.c_uint), ("lo_iterative_iterations", C.c_uint),
-                ("lo_threshold_multiplier", C.c_uint), ("max_hypothesis_test_before_sprt", C.c_uint)]
+                ("lo_threshold_multiplier", C.c_uint), ("max_hypothesis_test_before_sprt", C.c_uint), ("essential_roots", C.c_int)]
 
 
 class FitResult(C.Structure):
@@ -88,6 +90,7 @@ def load():
     L.usac_gpu_get_inliers.argtypes = [vp, C.c_int, fp, C.c_float, ip, ip]
     L.usac_gpu_sample.argtypes = [vp, C.c_int, C.POINTER(SamplerCfg), C.c_uint64, C.c_int, ip]
     L.usac_gpu_estimate.argtypes = [vp, C.c_int, ip, C.c_int, fp, ip]
+    L.usac_gpu_estimate_essential_roots.argtypes = [vp, C.c_int, ip, C.c_int, fp, ip]
     L.usac_gpu_fit.argtypes = [vp, C.POINTER(FitCfg), C.POINTER(FitResult)]
     L.usac_gpu_estimate_nonminimal.argtypes = [vp, C.c_int, ip, C.c_int, fp, ip]
     L.usac_gpu_refit.argtypes = [vp, C.c_int, fp, C.c_int, C.c_float, C.POINTER(RefitResult)]

@@ -436,8 +436,9 @@ __device__ bool stage_root(const double (*C)[20], const double (*L)[4], const do
 
 }  // namespace e5
 
-// one thread per sample
-__device__ __noinline__ int solve_essential5(const float* __restrict__ pts, const int* s, float* out) {
+// one thread per sample. all_roots = 0: the first root that passes the cheirality vote (the reference's rule), out[9];
+// all_roots = 1: every such root in visiting order, out[k * 9], k <= 10
+__device__ __noinline__ int solve_essential5(const float* __restrict__ pts, const int* s, float* out, int all_roots) {
     using namespace e5;
     double X[20], L[9][4], C[10][20];
     if (!stage_constraints(pts, s, X, L, C)) return 0;
@@ -453,20 +454,23 @@ __device__ __noinline__ int solve_essential5(const float* __restrict__ pts, cons
         nroots = stage_collect(pass, rr, nr, roots, nroots);
     }
     stage_sort(roots, nroots);
+    int k = 0;
     for (int ri = 0; ri < nroots; ri++) {
         double E[9];
         if (stage_root(C, L, X, roots[ri], E)) {
-            for (int e = 0; e < 9; e++) out[e] = (float)E[e];
-            return 1;
+            for (int e = 0; e < 9; e++) out[9 * k + e] = (float)E[e];
+            k++;
+            if (!all_roots) break;
         }
     }
-    return 0;
+    return k;
 }
 
 // one warp per sample: `sm` points to E5_WARP_DOUBLES doubles of shared memory owned by this warp. Every lane returns the
-// model count; lane 0 .. (the lane that owns the winning root) writes `out`.
+// model count; the lane that owns the winning root writes `out` (all_roots: every lane with a valid root writes its E at
+// out + 9 * (valid roots of the lanes below it), so the models are compacted in visiting order).
 #define E5_WARP_DOUBLES (20 + 36 + 200 + 22 + 22 + 242 + 24 + 24 + 20 + 60 + 800)
-__device__ int solve_essential5_warp(const float* __restrict__ pts, const int* s, float* out, double* sm) {
+__device__ int solve_essential5_warp(const float* __restrict__ pts, const int* s, float* out, double* sm, int all_roots) {
     using namespace e5;
     const int lane = threadIdx.x & 31;
     double* X = sm;                                                    // 20
@@ -582,6 +586,13 @@ __device__ int solve_essential5_warp(const float* __restrict__ pts, const int* s
     const bool ok = alive && stage_root_finish(L, X, u, E);
     const unsigned win = __ballot_sync(0xffffffffu, ok);
     if (!win) return 0;
+    if (all_roots) {
+        if (ok) {
+            float* dst = out + 9 * __popc(win & ((1u << lane) - 1u));
+            for (int e = 0; e < 9; e++) dst[e] = (float)E[e];
+        }
+        return __popc(win);
+    }
     if (lane == __ffs(win) - 1) for (int e = 0; e < 9; e++) out[e] = (float)E[e];
     return 1;
 }

@@ -10,6 +10,8 @@ struct RoundArgs {
     FitState* state;             // per problem
     const float* aos;
     int est, K, S, m, mstride;   // samples per round, models per sample, sample size, K*S
+    int e5_all_roots;            // essential: every cheirality-valid root is a model (S = USAC_E5_MAX_ROOTS), else the first one
+    int midx_shift;              // per-sample score packing: model index above bit midx_shift (30: up to 3 models, 28: up to 10)
     // sampler
     int sampler, rng, neighbors;
     uint64_t seed;
@@ -28,7 +30,7 @@ struct RoundArgs {
     uint2* items;                // compact work-item list of the scoring kernel: (slot, chunk << 16 | model group), only groups that hold models
     unsigned* item_count;        // [0] = number of items (zeroed by the host before the round), [1] = the scoring kernel's draw counter
     int* part_cnt; float* part_sum; int nchunks;   // [nchunks][K*S]
-    uint2* sample_scores;        // [K] per-sample best (cnt | midx<<30, sum bits); with nranks>1: [nranks][ceil(K/nranks)]
+    uint2* sample_scores;        // [K] per-sample best (cnt | midx << midx_shift, sum bits); with nranks>1: [nranks][ceil(K/nranks)]
     // fit parameters
     float thr, confidence;
     unsigned max_iterations;
@@ -383,21 +385,23 @@ __global__ void __launch_bounds__(32 * E5_WARPS_PER_CTA, E5_MIN_CTAS) solve_kern
     const int* src = a.samples + ((size_t)slot * a.K + j) * a.m;
     for (int i = 0; i < a.m; i++) s[i] = src[i];
     float* dst = a.models_raw + ((size_t)slot * a.K + j) * a.S * 9;
-    const int k = solve_essential5_warp(pts, s, dst, sm[w]);
+    const int k = solve_essential5_warp(pts, s, dst, sm[w], a.e5_all_roots);
     if (lane == 0) *nm = k;
 }
+// S = 1: the first valid root per sample (usac_gpu_estimate); S = USAC_E5_MAX_ROOTS with all_roots (usac_gpu_estimate_essential_roots)
 __global__ void __launch_bounds__(32 * E5_WARPS_PER_CTA, E5_MIN_CTAS) estimate_kernel_e5_warp(const float* __restrict__ pts, const int* __restrict__ samples, int K,
-                                                                                float* __restrict__ models, int* __restrict__ nmodels) {
+                                                                                int S, int all_roots, float* __restrict__ models,
+                                                                                int* __restrict__ nmodels) {
     __shared__ double sm[E5_WARPS_PER_CTA][E5_WARP_DOUBLES];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int j = blockIdx.x * E5_WARPS_PER_CTA + w;
     if (j >= K) return;
     int s[8];
     for (int i = 0; i < 5; i++) s[i] = samples[(size_t)j * 5 + i];
-    float* dst = models + (size_t)j * 9;
-    if (lane < 9) dst[lane] = 0.f;
+    float* dst = models + (size_t)j * S * 9;
+    for (int i = lane; i < S * 9; i += 32) dst[i] = 0.f;
     __syncwarp();
-    const int k = solve_essential5_warp(pts, s, dst, sm[w]);
+    const int k = solve_essential5_warp(pts, s, dst, sm[w], all_roots);
     if (lane == 0) nmodels[j] = k;
 }
 
@@ -465,7 +469,8 @@ __global__ void __launch_bounds__(1024) prepare_kernel(const RoundArgs a) {
     }
     if (threadIdx.x == 0) a.mvalid[slot] = total;
     // Work items of the scoring kernel for this slot: (point chunk, group of 32 models) for the groups that exist. Fundamental
-    // matrices pass the oriented-epipolar filter for a fraction of the samples only, the five-point solver returns 0 or 1 model:
+    // matrices pass the oriented-epipolar filter for a fraction of the samples only, the five-point solver returns 0 or 1 model
+    // (0..10 with e5_all_roots, 0.44 per sample on C4):
     // a grid over K x S model slots would be mostly empty groups.
     if (a.items) {
         __shared__ unsigned s_base;
@@ -483,6 +488,12 @@ __global__ void __launch_bounds__(1024) prepare_kernel(const RoundArgs a) {
 __device__ __forceinline__ bool score_bigger(int ca, float sa, int cb, float sb) {   // Score::bigger, quality.hpp:22-26
     return ca > cb || (ca == cb && sa > sb);
 }
+// Per-sample score word: the inlier count below bit midx_shift, the index of the sample's best model above it; the field's
+// all-ones value marks a sample without a model. Counts of an all-roots fit are < 2^28 (usac_gpu_fit checks n).
+__device__ __forceinline__ unsigned pack_cnt_midx(const RoundArgs& a, int cnt, int midx) { return (unsigned)cnt | ((unsigned)midx << a.midx_shift); }
+__device__ __forceinline__ int packed_cnt(const RoundArgs& a, unsigned x) { return (int)(x & ((1u << a.midx_shift) - 1u)); }
+__device__ __forceinline__ int packed_midx(const RoundArgs& a, unsigned x) { return (int)(x >> a.midx_shift); }
+__device__ __forceinline__ int midx_none(const RoundArgs& a) { return (int)(0xffffffffu >> a.midx_shift); }
 
 __global__ void reduce_kernel(const RoundArgs a) {
     const int slot = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -501,10 +512,10 @@ __global__ void reduce_kernel(const RoundArgs a) {
             }
             if (bc < 0 || score_bigger(c, s, bc, bs)) { bc = c; bs = s; bi = i; }
         }
-        if (bc < 0) { bc = 0; bs = 0.f; bi = 3; }                       // no model: midx 3 marks "nothing to compare"
+        if (bc < 0) { bc = 0; bs = 0.f; bi = midx_none(a); }             // no model: "nothing to compare"
         const int per_rank = (a.K + a.nranks - 1) / a.nranks;
         const size_t dst = (a.nranks > 1) ? ((size_t)slot * per_rank + j / a.nranks) : ((size_t)slot * a.K + j);
-        const uint2 v = make_uint2((unsigned)bc | ((unsigned)bi << 30), __float_as_uint(bs));
+        const uint2 v = make_uint2(pack_cnt_midx(a, bc, bi), __float_as_uint(bs));
         if (a.peer_win) peer_store(a, (size_t)a.rank * gridDim.y * per_rank + dst, v);
         else a.sample_scores[dst] = v;
     }
@@ -513,17 +524,18 @@ __global__ void reduce_kernel(const RoundArgs a) {
 
 // The same for many point chunks (one large problem: hundreds of partials per model): a CTA of 8 warps owns 32 samples
 // (lane <-> sample, coalesced), warp w sums the chunks w, w+8, ... and the eight partial sums are added in warp order
-// (fixed order -> deterministic).
+// (fixed order -> deterministic). SMAX >= a.S.
+template <int SMAX>
 __global__ void __launch_bounds__(256) reduce_chunks_kernel(const RoundArgs a) {
-    __shared__ int s_c[8][3][32];
-    __shared__ float s_s[8][3][32];
+    __shared__ int s_c[8][SMAX][32];
+    __shared__ float s_s[8][SMAX][32];
     const int slot = blockIdx.y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int own = blockIdx.x * 32 + lane;                            // this rank's samples, densely: j = own * nranks + rank
     const int j = a.nranks > 1 ? own * a.nranks + a.rank : own;
     const bool mine = j < a.K;
     const int k = mine ? a.nmodels[(size_t)slot * a.K + j] : 0;
     const int off = mine ? a.offsets[(size_t)slot * a.K + j] : 0;
-    for (int i = 0; i < 3; i++) {
+    for (int i = 0; i < SMAX; i++) {
         int c = 0;
         float s = 0.f;
         if (i < k)
@@ -545,10 +557,10 @@ __global__ void __launch_bounds__(256) reduce_chunks_kernel(const RoundArgs a) {
             for (int w = 0; w < 8; w++) { c += s_c[w][i][lane]; s += s_s[w][i][lane]; }
             if (bc < 0 || score_bigger(c, s, bc, bs)) { bc = c; bs = s; bi = i; }
         }
-        if (bc < 0) { bc = 0; bs = 0.f; bi = 3; }
+        if (bc < 0) { bc = 0; bs = 0.f; bi = midx_none(a); }
         const int per_rank = (a.K + a.nranks - 1) / a.nranks;
         const size_t dst = (a.nranks > 1) ? ((size_t)slot * per_rank + own) : ((size_t)slot * a.K + j);
-        const uint2 v = make_uint2((unsigned)bc | ((unsigned)bi << 30), __float_as_uint(bs));
+        const uint2 v = make_uint2(pack_cnt_midx(a, bc, bi), __float_as_uint(bs));
         if (a.peer_win) peer_store(a, (size_t)a.rank * gridDim.y * per_rank + dst, v);
         else a.sample_scores[dst] = v;
     }
@@ -587,14 +599,15 @@ __global__ void __launch_bounds__(256) select_kernel(const RoundArgs a, const ui
     };
     const unsigned long long carry_key = score_key(st.best_cnt, st.best_sum);
     const unsigned iters0 = st.iters, carry_max = st.max_iters;
+    const int none = midx_none(a);
 
     const int per = (K + blockDim.x - 1) / blockDim.x;
     const int j0 = threadIdx.x * per, j1 = min(j0 + per, K);
     SelKey mine = {0ull, -1};
     for (int j = j0; j < j1; j++) {
         const uint2 v = load(j);
-        if ((v.x >> 30) == 3u) continue;
-        SelKey c = {score_key((int)(v.x & 0x3fffffffu), __uint_as_float(v.y)), j};
+        if (packed_midx(a, v.x) == none) continue;
+        SelKey c = {score_key(packed_cnt(a, v.x), __uint_as_float(v.y)), j};
         mine = sel_max(mine, c);
     }
     // exclusive prefix over threads of the "leftmost maximum" (associative): shuffle scan inside each warp, then the
@@ -619,7 +632,7 @@ __global__ void __launch_bounds__(256) select_kernel(const RoundArgs a, const ui
     SelKey at_stop = run;
     for (int j = j0; j < j1; j++) {
         const uint2 v = load(j);
-        if ((v.x >> 30) != 3u) { SelKey c = {score_key((int)(v.x & 0x3fffffffu), __uint_as_float(v.y)), j}; run = sel_max(run, c); }
+        if (packed_midx(a, v.x) != none) { SelKey c = {score_key(packed_cnt(a, v.x), __uint_as_float(v.y)), j}; run = sel_max(run, c); }
         const unsigned mi = (run.j < 0) ? carry_max : table[(unsigned)(run.key >> 32)];
         if (iters0 + (unsigned)j + 1u >= mi) { stop = j; at_stop = run; break; }
     }
@@ -651,10 +664,10 @@ __global__ void __launch_bounds__(256) select_kernel(const RoundArgs a, const ui
         const SelKey best = (T < K) ? at_stop : run;
         if (best.j >= 0) {
             const uint2 v = load(best.j);
-            st.best_cnt = (int)(v.x & 0x3fffffffu);
+            st.best_cnt = packed_cnt(a, v.x);
             st.best_sum = __uint_as_float(v.y);
             st.best_hyp = (long long)st.samples_drawn + best.j;
-            st.best_midx = (int)(v.x >> 30);
+            st.best_midx = packed_midx(a, v.x);
             st.max_iters = table[(unsigned)st.best_cnt];
         }
         st.iters = iters0 + (unsigned)min(T + 1, K);
@@ -688,9 +701,9 @@ __global__ void winner_kernel(const RoundArgs a, int slots) {
             int s[8];
             const int* src = a.samples + ((size_t)slot * a.K + j) * a.m;
             for (int i = 0; i < a.m; i++) s[i] = src[i];
-            float out[27];
+            float out[EST == USAC_EST_ESSENTIAL ? 9 * USAC_E5_MAX_ROOTS : 27];
             const float* pts = a.aos + (size_t)pd.aos_off * (EST == USAC_EST_LINE2D ? 2 : 4);
-            const int k = solve_minimal<EST>(pts, s, out);
+            const int k = solve_minimal<EST>(pts, s, out, a.e5_all_roots);
             if (st.best_midx < k) for (int i = 0; i < w; i++) st.best_model[i] = out[9 * st.best_midx + i];
         }
     }

@@ -379,12 +379,13 @@ __device__ int solve_fundamental7(const float* __restrict__ pts, const int* s, f
     return valid;
 }
 
-__device__ int solve_essential5(const float* __restrict__ pts, const int* s, float* out);   // essential.cuh
+__device__ int solve_essential5(const float* __restrict__ pts, const int* s, float* out, int all_roots);   // essential.cuh
 
+// out: up to 3 models (fundamental), up to USAC_E5_MAX_ROOTS with e5_all_roots, else one
 template <int EST>
-__device__ __forceinline__ int solve_minimal(const float* __restrict__ pts, const int* s, float* out) {
+__device__ __forceinline__ int solve_minimal(const float* __restrict__ pts, const int* s, float* out, int e5_all_roots = 0) {
     if (EST == USAC_EST_LINE2D) return solve_line2d(pts, s, out);
     if (EST == USAC_EST_HOMOGRAPHY) return solve_homography4(pts, s, out);
     if (EST == USAC_EST_FUNDAMENTAL) return solve_fundamental7(pts, s, out);
-    return solve_essential5(pts, s, out);
+    return solve_essential5(pts, s, out, e5_all_roots);
 }

@@ -1020,8 +1020,13 @@ static void prosac_growth(unsigned n, unsigned m, std::vector<unsigned>& g) {
 // ------------------------------------------------------------------------------------------------------------------
 // Sampler / Estimator APIs
 // ------------------------------------------------------------------------------------------------------------------
-static int ensure_round_buffers(usac_gpu_ctx* c, int slots, int K, int nchunks, int nranks) {
-    const int S = usac_models_per_sample(c->est), m = usac_sample_size(c->est);
+// models per sample of a fit: the solver's maximum, or USAC_E5_MAX_ROOTS for an essential fit that keeps every valid root
+static int fit_models_per_sample(int est, const usac_fit_cfg* cfg) {
+    return cfg->essential_roots == USAC_E5_ROOTS_ALL_VALID ? USAC_E5_MAX_ROOTS : usac_models_per_sample(est);
+}
+
+static int ensure_round_buffers(usac_gpu_ctx* c, int slots, int K, int nchunks, int nranks, int S) {
+    const int m = usac_sample_size(c->est);
     const size_t sk = (size_t)slots * K;
     CUDA_TRY(c, c->d_samples.ensure(sk * m));
     CUDA_TRY(c, c->d_nmodels.ensure(sk));
@@ -1067,10 +1072,12 @@ static int setup_sampler_side(usac_gpu_ctx* c, const usac_sampler_cfg& s, bool r
     return USAC_OK;
 }
 
-static void fill_round_args(usac_gpu_ctx* c, RoundArgs& a, const usac_sampler_cfg& s, int K) {
+static void fill_round_args(usac_gpu_ctx* c, RoundArgs& a, const usac_sampler_cfg& s, int K, int S) {
     memset(&a, 0, sizeof(a));
     a.prob = c->d_prob.p; a.active = c->d_active.p; a.state = c->d_state.p; a.aos = c->d_aos.p;
-    a.est = c->est; a.K = K; a.S = usac_models_per_sample(c->est); a.m = usac_sample_size(c->est); a.mstride = K * a.S;
+    a.est = c->est; a.K = K; a.S = S; a.m = usac_sample_size(c->est); a.mstride = K * a.S;
+    a.e5_all_roots = c->est == USAC_EST_ESSENTIAL && S == USAC_E5_MAX_ROOTS;
+    a.midx_shift = S > 3 ? 28 : 30;
     a.sampler = s.sampler; a.rng = s.rng; a.neighbors = s.neighbors; a.seed = s.seed;
     a.growth = c->d_growth.p; a.knn = c->d_knn.p; a.cell_of_point = c->d_cell_of_point.p; a.members = c->d_members.p;
     a.rank_in_cell = c->d_rank.p; a.cell_start = c->d_cell_start.p; a.cursors = c->d_cursors.p; a.seeds = c->d_seeds.p;
@@ -1115,7 +1122,7 @@ extern "C" int usac_gpu_sample(usac_gpu_ctx* c, int problem, const usac_sampler_
     if (const char* why = check_sampler_cfg(*cfg)) return fail(c, USAC_ERR_ARG, why);
     if (cfg->rng == USAC_RNG_TABLE) return fail(c, USAC_ERR_ARG, "sample: table replay has nothing to generate");
     cudaSetDevice(c->device);
-    int rc = ensure_round_buffers(c, 1, K, 1, 1);
+    int rc = ensure_round_buffers(c, 1, K, 1, 1, usac_models_per_sample(c->est));
     if (rc) return rc;
     rc = setup_sampler_side(c, *cfg, first_hyp == 0);   // NAPSAC cursors persist across calls that continue a stream
     if (rc) return rc;
@@ -1139,7 +1146,7 @@ extern "C" int usac_gpu_sample(usac_gpu_ctx* c, int problem, const usac_sampler_
     c->h_active[0] = problem;
     CUDA_TRY(c, cudaMemcpyAsync(c->d_active.p, c->h_active, sizeof(int), cudaMemcpyHostToDevice, c->stream));
     RoundArgs a;
-    fill_round_args(c, a, *cfg, K);
+    fill_round_args(c, a, *cfg, K, usac_models_per_sample(c->est));
     c->last_launches = 0;
     launch_sampler(c, a, 1);
     CUDA_TRY(c, cudaMemcpyAsync(samples_out, c->d_samples.p, sizeof(int) * K * a.m, cudaMemcpyDeviceToHost, c->stream));
@@ -1148,10 +1155,10 @@ extern "C" int usac_gpu_sample(usac_gpu_ctx* c, int problem, const usac_sampler_
     return USAC_OK;
 }
 
-extern "C" int usac_gpu_estimate(usac_gpu_ctx* c, int problem, const int* samples, int K, float* models_out, int* nmodels_out) {
-    if (!c || problem < 0 || problem >= c->P || !samples || K <= 0 || !models_out || !nmodels_out) return fail(c, USAC_ERR_ARG, "estimate: bad arguments");
+// S models per sample in models_out: usac_models_per_sample, or USAC_E5_MAX_ROOTS with e5_all_roots
+static int estimate_models(usac_gpu_ctx* c, int problem, const int* samples, int K, float* models_out, int* nmodels_out, bool e5_all_roots) {
     cudaSetDevice(c->device);
-    const int S = usac_models_per_sample(c->est), m = usac_sample_size(c->est), dim = usac_point_dim(c->est);
+    const int S = e5_all_roots ? USAC_E5_MAX_ROOTS : usac_models_per_sample(c->est), m = usac_sample_size(c->est), dim = usac_point_dim(c->est);
     const ProblemDesc& d = c->h_prob[problem];
     for (size_t i = 0; i < (size_t)K * m; i++)
         if (samples[i] < 0 || samples[i] >= d.n) return fail(c, USAC_ERR_ARG, "estimate: sample index out of range");
@@ -1165,13 +1172,27 @@ extern "C" int usac_gpu_estimate(usac_gpu_ctx* c, int problem, const int* sample
         case USAC_EST_LINE2D: estimate_kernel<USAC_EST_LINE2D><<<g, 64, 0, c->stream>>>(aos, c->d_samples.p, K, m, S, c->d_models_raw.p, c->d_nmodels.p); break;
         case USAC_EST_HOMOGRAPHY: estimate_kernel<USAC_EST_HOMOGRAPHY><<<g, 64, 0, c->stream>>>(aos, c->d_samples.p, K, m, S, c->d_models_raw.p, c->d_nmodels.p); break;
         case USAC_EST_FUNDAMENTAL: estimate_kernel<USAC_EST_FUNDAMENTAL><<<g, 64, 0, c->stream>>>(aos, c->d_samples.p, K, m, S, c->d_models_raw.p, c->d_nmodels.p); break;
-        default: estimate_kernel_e5_warp<<<(K + E5_WARPS_PER_CTA - 1) / E5_WARPS_PER_CTA, 32 * E5_WARPS_PER_CTA, 0, c->stream>>>(aos, c->d_samples.p, K, c->d_models_raw.p, c->d_nmodels.p); break;
+        default:
+            estimate_kernel_e5_warp<<<(K + E5_WARPS_PER_CTA - 1) / E5_WARPS_PER_CTA, 32 * E5_WARPS_PER_CTA, 0, c->stream>>>(aos, c->d_samples.p, K, S, e5_all_roots ? 1 : 0,
+                                                                                                                c->d_models_raw.p, c->d_nmodels.p);
+            break;
     }
     CUDA_TRY(c, cudaMemcpyAsync(models_out, c->d_models_raw.p, sizeof(float) * K * S * 9, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaMemcpyAsync(nmodels_out, c->d_nmodels.p, sizeof(int) * K, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     CUDA_TRY(c, cudaGetLastError());
     return USAC_OK;
+}
+
+extern "C" int usac_gpu_estimate(usac_gpu_ctx* c, int problem, const int* samples, int K, float* models_out, int* nmodels_out) {
+    if (!c || problem < 0 || problem >= c->P || !samples || K <= 0 || !models_out || !nmodels_out) return fail(c, USAC_ERR_ARG, "estimate: bad arguments");
+    return estimate_models(c, problem, samples, K, models_out, nmodels_out, false);
+}
+
+extern "C" int usac_gpu_estimate_essential_roots(usac_gpu_ctx* c, int problem, const int* samples, int K, float* models_out, int* nmodels_out) {
+    if (!c || problem < 0 || problem >= c->P || !samples || K <= 0 || !models_out || !nmodels_out) return fail(c, USAC_ERR_ARG, "estimate_essential_roots: bad arguments");
+    if (c->est != USAC_EST_ESSENTIAL) return fail(c, USAC_ERR_ARG, "estimate_essential_roots: the uploaded points are not an essential problem");
+    return estimate_models(c, problem, samples, K, models_out, nmodels_out, true);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -1464,11 +1485,11 @@ __global__ void gather_models_kernel(const float* __restrict__ models_raw, const
 // it needs libm for the SPRT bound) and the models of the new best hypotheses come back through one gather. Per problem the
 // result is that of the one-problem-at-a-time path (rounds of K, test frozen within a round).
 static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_result* results, int K) {
-    const int P = c->P, m = usac_sample_size(c->est), S = usac_models_per_sample(c->est), w = c->est == USAC_EST_LINE2D ? 3 : 9;
+    const int P = c->P, m = usac_sample_size(c->est), S = fit_models_per_sample(c->est, cfg), w = c->est == USAC_EST_LINE2D ? 3 : 9;
     const float log_1_p = (float)logf(1 - cfg->confidence);
     const int KS = K * S;
     const unsigned before_sprt = cfg->max_hypothesis_test_before_sprt ? cfg->max_hypothesis_test_before_sprt : 20u;
-    int rc = ensure_round_buffers(c, P, K, 1, 1);
+    int rc = ensure_round_buffers(c, P, K, 1, 1, S);
     if (rc) return rc;
     CUDA_TRY(c, c->h_rp_nmodels.ensure((size_t)P * K));
     CUDA_TRY(c, c->h_rp_res.ensure((size_t)P * KS));
@@ -1495,7 +1516,7 @@ static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_res
         CUDA_TRY(c, cudaMemcpyAsync(c->d_state.p, c->h_state, sizeof(FitState) * P, cudaMemcpyHostToDevice, c->stream));
         CUDA_TRY(c, cudaMemcpyAsync(c->d_active.p, c->h_active, sizeof(int) * slots, cudaMemcpyHostToDevice, c->stream));
         RoundArgs a;
-        fill_round_args(c, a, cfg->sampler, K);
+        fill_round_args(c, a, cfg->sampler, K, S);
         a.thr = cfg->threshold; a.confidence = cfg->confidence; a.max_iterations = cfg->max_iterations;
         a.table_rows = cfg->sample_table_rows; a.nchunks = 1; a.sprt = cfg->sprt; a.pool = c->d_pool.p; a.sprt_res = c->d_sprt_res.p;
         a.before_sprt = before_sprt;
@@ -1609,7 +1630,7 @@ static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_res
 }
 
 static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_result* results, int K) {
-    const int P = c->P, m = usac_sample_size(c->est), S = usac_models_per_sample(c->est), w = c->est == USAC_EST_LINE2D ? 3 : 9;
+    const int P = c->P, m = usac_sample_size(c->est), S = fit_models_per_sample(c->est, cfg), w = c->est == USAC_EST_LINE2D ? 3 : 9;
     const bool is_prosac = cfg->sampler.sampler == USAC_SAMPLER_PROSAC, is_sprt = cfg->sprt != 0;
     const float log_1_p = (float)logf(1 - cfg->confidence);
     const int KS = K * S;
@@ -1630,7 +1651,7 @@ static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_re
     // ... and the NEXT block is solved on a second stream while this block's rounds run (walks, copies, the host replay): two sets of
     // sample / model / record buffers, used alternately
     const bool overlap = G > 1 && !(getenv("USAC_GPU_SOLVE_OVERLAP") && atoi(getenv("USAC_GPU_SOLVE_OVERLAP")) == 0);
-    int rc = ensure_round_buffers(c, 1, overlap ? 2 * KB : KB, 1, 1);
+    int rc = ensure_round_buffers(c, 1, overlap ? 2 * KB : KB, 1, 1, S);
     if (rc) return rc;
     if (overlap && !c->stream2) {
         CUDA_TRY(c, cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking));
@@ -1686,7 +1707,7 @@ static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_re
             const int mblocks = (KS + USAC_SCORE_THREADS - 1) / USAC_SCORE_THREADS;
             if (!is_sprt) {
                 plan_chunks(c, 1, mblocks, pd.n_pairs, &chunk_pairs, &nchunks);
-                rc = ensure_round_buffers(c, 1, K, nchunks, 1);
+                rc = ensure_round_buffers(c, 1, K, nchunks, 1, S);
                 if (rc) return rc;
             }
             if (overlap) CUDA_TRY(c, cudaEventRecord(c->ev_round, c->stream));   // everything up to this round's state upload
@@ -1696,7 +1717,7 @@ static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_re
             const int blk = block_round / G, par = overlap ? (blk & 1) : 0;
             auto launch_block = [&](int parity, unsigned long long hyp_base_p1) {   // sample + solve + records of one block of G rounds
                 RoundArgs b;
-                fill_round_args(c, b, cfg->sampler, KB);
+                fill_round_args(c, b, cfg->sampler, KB, S);
                 b.thr = cfg->threshold; b.confidence = cfg->confidence; b.max_iterations = cfg->max_iterations;
                 b.table_rows = cfg->sample_table_rows; b.nchunks = nchunks; b.sprt = cfg->sprt; b.pool = c->d_pool.p; b.sprt_res = c->d_sprt_res.p;
                 b.before_sprt = before_sprt;
@@ -1740,7 +1761,7 @@ static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_re
             block_round++;
             // this round's view of the block: samples [g K, (g + 1) K); record offsets stay relative to the block
             RoundArgs a;
-            fill_round_args(c, a, cfg->sampler, K);
+            fill_round_args(c, a, cfg->sampler, K, S);
             a.thr = cfg->threshold; a.confidence = cfg->confidence; a.max_iterations = cfg->max_iterations;
             a.table_rows = cfg->sample_table_rows; a.nchunks = nchunks; a.sprt = cfg->sprt; a.pool = c->d_pool.p; a.sprt_res = c->d_sprt_res.p;
             a.before_sprt = before_sprt;
@@ -1915,6 +1936,9 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
     if (cfg->sampler.rng == USAC_RNG_TABLE && (!cfg->sample_table || cfg->sample_table_rows == 0)) return fail(c, USAC_ERR_ARG, "fit: empty sample table");
     if (cfg->lo != 0 && cfg->lo != 1 && cfg->lo != 2) return fail(c, USAC_ERR_ARG, "fit: lo must be 0 (none), 1 (InItLORsc) or 2 (InItFLORsc); GC / IRLS are not built");
     if (cfg->lo && c->est == USAC_EST_LINE2D) return fail(c, USAC_ERR_ARG, "fit: local optimisation of line models is not built");
+    if (cfg->essential_roots != USAC_E5_ROOTS_FIRST_VALID && cfg->essential_roots != USAC_E5_ROOTS_ALL_VALID)
+        return fail(c, USAC_ERR_ARG, "fit: essential_roots must be USAC_E5_ROOTS_FIRST_VALID or USAC_E5_ROOTS_ALL_VALID");
+    if (cfg->essential_roots && c->est != USAC_EST_ESSENTIAL) return fail(c, USAC_ERR_ARG, "fit: essential_roots applies to essential fits only");
     if (cfg->lo && cfg->lo_sample_size && (cfg->lo_sample_size < (unsigned)usac_sample_size(c->est) + 1 || cfg->lo_sample_size > 16))
         return fail(c, USAC_ERR_ARG, "fit: lo_sample_size must lie in [sample size + 1, 16]");
     const bool host_replay = cfg->sprt || cfg->lo || cfg->sampler.sampler == USAC_SAMPLER_PROSAC;
@@ -1931,9 +1955,10 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
     const auto t_begin = now();
     double t_enqueue = 0, t_wait = 0;
     int n_rounds = 0;
-    const int P = c->P, m = usac_sample_size(c->est), S = usac_models_per_sample(c->est);
+    const int P = c->P, m = usac_sample_size(c->est), S = fit_models_per_sample(c->est, cfg);
     int max_n = 0;
     for (int p = 0; p < P; p++) max_n = std::max(max_n, c->h_prob[p].n);
+    if (S > 3 && max_n >= (1 << 28)) return fail(c, USAC_ERR_ARG, "fit: USAC_E5_ROOTS_ALL_VALID needs fewer than 2^28 points per problem");
     if (cfg->sprt) for (int p = 0; p < P; p++) if (!c->h_pool_set[p]) return fail(c, USAC_ERR_STATE, "fit: SPRT needs usac_gpu_set_sprt_pool for every problem");
 
     int K = cfg->round_size;
@@ -2043,10 +2068,10 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
         // the seven-point solver after the oriented-epipolar filter (0..3 models)
         const int expect_models = (c->est == USAC_EST_FUNDAMENTAL || c->est == USAC_EST_ESSENTIAL) ? (K + 1) / 2 : K;
         plan_chunks(c, slots, std::max(1, ((expect_models + USAC_SCORE_THREADS - 1) / USAC_SCORE_THREADS) / nranks), max_pairs, &chunk_pairs, &nchunks);
-        rc = ensure_round_buffers(c, slots, K, nchunks, nranks);
+        rc = ensure_round_buffers(c, slots, K, nchunks, nranks, S);
         if (rc) return rc;
         RoundArgs a;
-        fill_round_args(c, a, cfg->sampler, K);
+        fill_round_args(c, a, cfg->sampler, K, S);
         a.active = act_cur;
         a.thr = cfg->threshold; a.confidence = cfg->confidence; a.max_iterations = cfg->max_iterations;
         a.table_rows = cfg->sample_table_rows; a.rank = rank; a.nranks = nranks; a.nchunks = nchunks;
@@ -2092,7 +2117,9 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
                 TK("score");
                 dim3 gr((K + 127) / 128, slots);
                 if (use_peer) { a.peer_seq = ++c->peer_seq; c->peer_rounds++; }
-                if (nchunks > 8) reduce_chunks_kernel<<<dim3(((K + nranks - 1) / nranks + 31) / 32, slots), 256, 0, c->stream>>>(a);
+                const dim3 grc_grid(((K + nranks - 1) / nranks + 31) / 32, slots);
+                if (nchunks > 8 && S > 3) reduce_chunks_kernel<USAC_E5_MAX_ROOTS><<<grc_grid, 256, 0, c->stream>>>(a);
+                else if (nchunks > 8) reduce_chunks_kernel<USAC_MAX_MODELS_PER_SAMPLE><<<grc_grid, 256, 0, c->stream>>>(a);
                 else reduce_kernel<<<gr, 128, 0, c->stream>>>(a);
                 c->last_launches++;
                 const uint2* scores = c->d_scores.p;

@@ -70,7 +70,8 @@ private:
     static std::map<const float*, GpuDevice*>& registry() { static std::map<const float*, GpuDevice*> r; return r; }
 };
 
-// Estimator (estimator.hpp:19-40): EstimateModel = the device minimal solver on one sample (usac_gpu_estimate, K = 1);
+// Estimator (estimator.hpp:19-40): EstimateModel = the device minimal solver on one sample (usac_gpu_estimate, K = 1;
+// usac_gpu_estimate_essential_roots when the models carry Model::gpu_essential_all_roots);
 // setModelParameters + GetError(pidx) = usac_gpu_errors (all N errors in the reference's exact arithmetic, cached).
 class GpuEstimator : public Estimator {
     GpuDevice* dev;
@@ -83,9 +84,12 @@ public:
     ~GpuEstimator() override { if (owns_device) delete dev; }
     int SampleNumber() override { return dev->estimator == USAC_EST_LINE2D ? 2 : dev->estimator == USAC_EST_HOMOGRAPHY ? 4 : dev->estimator == USAC_EST_FUNDAMENTAL ? 7 : 5; }
     unsigned int EstimateModel(const int* const sample, std::vector<Model*>& models) override {
-        float out[USAC_MAX_MODELS_PER_SAMPLE * 9];
+        float out[USAC_E5_MAX_ROOTS * 9];
         int n = 0;
-        dev->check(usac_gpu_estimate(dev->ctx, 0, sample, 1, out, &n), "usac_gpu_estimate");
+        if (dev->estimator == USAC_EST_ESSENTIAL && !models.empty() && models[0]->gpu_essential_all_roots)
+            dev->check(usac_gpu_estimate_essential_roots(dev->ctx, 0, sample, 1, out, &n), "usac_gpu_estimate_essential_roots");
+        else
+            dev->check(usac_gpu_estimate(dev->ctx, 0, sample, 1, out, &n), "usac_gpu_estimate");
         const bool line = dev->estimator == USAC_EST_LINE2D;
         for (int i = 0; i < n && i < (int)models.size(); i++) {
             cv::Mat d = line ? cv::Mat(1, 3) : cv::Mat(3, 3);

@@ -29,9 +29,11 @@ public:
     int cell_size = 50;
     bool reset_random_generator = true;
     std::string img_name;
-    // additions of the GPU host layer (not in the reference): explicit sampler seed and round size of the fused loop
+    // additions of the GPU host layer (not in the reference): explicit sampler seed and round size of the fused loop, and
+    // (essential only) every cheirality-valid five-point root as a model instead of the reference's first one
     unsigned long long seed = 1;
     int gpu_round_size = 0;
+    bool gpu_essential_all_roots = false;
 
     Model(const Model* const other) { copyFrom(other); }
     Model(float threshold_, unsigned int sample_number_, float desired_prob_, unsigned int knn, ESTIMATOR estimator_, SAMPLER sampler_)
@@ -42,6 +44,7 @@ public:
     void setNeighborsType(NeighborsSearch t) { neighborsType = t; }
     void setCellSize(int c) { cell_size = c; }
     void setSprt(bool s) { sprt = s; }
+    void setGpuEssentialAllRoots(bool a) { gpu_essential_all_roots = a; }
     void setLOParametres(unsigned int it, unsigned int inner, unsigned int mult) {
         lo_iterative_iterations = it; lo_inner_iterations = inner; lo_threshold_multiplier = mult;
     }
@@ -59,7 +62,7 @@ public:
         lo_threshold_multiplier = m->lo_threshold_multiplier; reset_random_generator = m->reset_random_generator;
         lo = m->lo; sprt = m->sprt; spatial_coherence_gc = m->spatial_coherence_gc; cell_size = m->cell_size;
         neighborsType = m->neighborsType; max_hypothesis_test_before_sprt = m->max_hypothesis_test_before_sprt;
-        seed = m->seed; gpu_round_size = m->gpu_round_size;
+        seed = m->seed; gpu_round_size = m->gpu_round_size; gpu_essential_all_roots = m->gpu_essential_all_roots;
     }
 
 private:

@@ -8,6 +8,7 @@
 //   --gt-model F    3 x 3 ground-truth model (Reader::getMatrix3x3, the *_model.txt files): GT inliers = points under the threshold
 //   usac_harness <points file> <line2d|homography|fundamental|essential> <uniform|prosac|napsac> <threshold> <confidence> [seed]
 //                [--format F] [--gt-model file] [--read-only] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K]
+//                [--all-roots]
 //                [--report] [--runs N --csv out.csv [--gt-inliers G]]
 // --read-only parses the input, prints `read n=.. dim=.. checksum=.. flagged_inliers=..` and exits (no GPU needed).
 // Prints one `key=value` line per result (model as IEEE bit patterns, inlier ids as a hash) for the parity tests; --report adds the
@@ -64,7 +65,7 @@ static Stat stat_of(std::vector<double> v) {
 
 int main(int argc, char** argv) {
     if (argc < 6 || !std::strcmp(argv[1], "--help")) {
-        std::fprintf(stderr, "usage: %s <points.txt> <line2d|homography|fundamental|essential> <uniform|prosac|napsac> <threshold> <confidence> [seed] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K] [--report] [--runs N --csv out.csv [--gt-inliers G]]\n", argv[0]);
+        std::fprintf(stderr, "usage: %s <points.txt> <line2d|homography|fundamental|essential> <uniform|prosac|napsac> <threshold> <confidence> [seed] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K] [--all-roots] [--report] [--runs N --csv out.csv [--gt-inliers G]]\n", argv[0]);
         return argc < 2 ? 2 : (!std::strcmp(argv[1], "--help") ? 0 : 2);
     }
     const std::string est = argv[2], smp = argv[3];
@@ -129,6 +130,7 @@ int main(int argc, char** argv) {
         else if (!std::strcmp(argv[i], "--gt-inliers") && i + 1 < argc) gt_inliers = std::atoi(argv[++i]);
         else if (!std::strcmp(argv[i], "--knn") && i + 1 < argc) knn = std::atoi(argv[++i]);
         else if (!std::strcmp(argv[i], "--sprt")) model.setSprt(true);
+        else if (!std::strcmp(argv[i], "--all-roots")) model.setGpuEssentialAllRoots(true);   // essential: every cheirality-valid root
         else if (!std::strcmp(argv[i], "--round") && i + 1 < argc) model.gpu_round_size = std::atoi(argv[++i]);
         else if (!std::strcmp(argv[i], "--max-iter") && i + 1 < argc) model.max_iterations = (unsigned)std::atoi(argv[++i]);
         else if ((!std::strcmp(argv[i], "--format") || !std::strcmp(argv[i], "--gt-model")) && i + 1 < argc) i++;
