@@ -61,6 +61,9 @@ int usac_gpu_set_neighbors_knn(usac_gpu_ctx* ctx, int problem, const int* neighb
 int usac_gpu_build_neighbors_knn(usac_gpu_ctx* ctx, int problem, int k);
 /* copy the installed kNN table (n x k) back to the host; k_out receives k */
 int usac_gpu_get_neighbors_knn(usac_gpu_ctx* ctx, int problem, int* neighbors_out, int* k_out);
+/* Progressive NAPSAC: hypotheses 0 .. local_samples-1 of a fit or sample stream are local (DESIGN.md section 4.8), later ones are
+ * the uniform sampler's. 0 = the default, 20 n. Reset by usac_gpu_set_points, like the neighbourhoods. */
+int usac_gpu_set_pnapsac_length(usac_gpu_ctx* ctx, int problem, unsigned long long local_samples);
 /* SPRT's shuffled point pool (sprt.hpp:93-107); host-generated so that it can replay the reference's random() stream */
 int usac_gpu_set_sprt_pool(usac_gpu_ctx* ctx, int problem, const int* pool);
 
@@ -79,13 +82,17 @@ typedef struct {
     int sampler;                 /* USAC_SAMPLER_* */
     int rng;                     /* USAC_RNG_* */
     uint64_t seed;
-    int neighbors;               /* NAPSAC: USAC_NEIGH_* (set with usac_gpu_set_neighbors_*) */
+    int neighbors;               /* NAPSAC: USAC_NEIGH_* (set with usac_gpu_set_neighbors_*); Progressive NAPSAC: USAC_NEIGH_KNN */
     unsigned prosac_termination_length;   /* PROSAC: frozen for the call; 0 = n */
     unsigned prosac_hyp_count;            /* PROSAC: t of the first sample of this call (starts at 1) */
 } usac_sampler_cfg;
 /* samples_out: K x m int32 (m = 2/4/7/5), hypothesis ids first_hyp .. first_hyp+K-1. Samplers other than UNIFORM / NAPSAC /
- * PROSAC (the reference's ProgressiveNapsac is an unfinished stub, progressive_sampler.hpp:149-172; Evsac / ProsacNapsac are
- * not wired in init.cpp:23-50) and rng values other than USAC_RNG_* are rejected with USAC_ERR_ARG. */
+ * PROSAC / PROGRESSIVE_NAPSAC (Evsac / ProsacNapsac are not wired in init.cpp:23-50) and rng values other than USAC_RNG_* are
+ * rejected with USAC_ERR_ARG. PROGRESSIVE_NAPSAC is this library's definition (DESIGN.md section 4.8; the reference's
+ * progressive_sampler.hpp:149-172 is an unfinished stub): a centre point per hypothesis, drawn from a neighbourhood of its kNN
+ * list that grows with the centre's uses, then uniform sampling from hypothesis usac_gpu_set_pnapsac_length on. It needs
+ * neighbors = USAC_NEIGH_KNN (else USAC_ERR_ARG) and an installed kNN table (else USAC_ERR_STATE). NAPSAC and Progressive NAPSAC
+ * are stateful: a call with first_hyp == 0 starts the stream afresh, a later call continues it. */
 int usac_gpu_sample(usac_gpu_ctx* ctx, int problem, const usac_sampler_cfg* cfg, uint64_t first_hyp, int K, int* samples_out);
 
 /* ---- Estimator: replaces Estimator::EstimateModel x K (estimator.hpp:19; line2d/homography/fundamental/essential) */

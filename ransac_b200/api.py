@@ -11,7 +11,7 @@ import numpy as np
 from . import capi
 from .capi import (E5_MAX_ROOTS, E5_ROOTS_ALL_VALID, E5_ROOTS_FIRST_VALID, EST_ESSENTIAL, EST_FUNDAMENTAL,  # noqa: F401
                    EST_HOMOGRAPHY, EST_LINE2D, MAX_MODELS, NEIGH_GRID, NEIGH_KNN, NEIGH_NONE, RNG_PHILOX, RNG_TABLE, SAMPLE_SIZE,
-                   SAMPLER_NAPSAC, SAMPLER_PROSAC, SAMPLER_UNIFORM)
+                   SAMPLER_NAPSAC, SAMPLER_PROGRESSIVE_NAPSAC, SAMPLER_PROSAC, SAMPLER_UNIFORM)
 
 
 class UsacGpuError(RuntimeError):
@@ -93,6 +93,10 @@ class GpuContext:
         k = C.c_int()
         self._check(self.L.usac_gpu_get_neighbors_knn(self.h, problem, _ptr(out, C.c_int), C.byref(k)), "get_neighbors_knn")
         return out.reshape(-1)[:int(self.n[problem]) * k.value].reshape(int(self.n[problem]), k.value).copy()
+
+    def set_pnapsac_length(self, problem, local_samples):
+        """Progressive NAPSAC: hypotheses from local_samples on are sampled uniformly (0 = the default, 20 n)."""
+        self._check(self.L.usac_gpu_set_pnapsac_length(self.h, problem, int(local_samples)), "set_pnapsac_length")
 
     def set_sprt_pool(self, problem, pool):
         t = np.ascontiguousarray(pool, dtype=np.int32)

@@ -84,6 +84,7 @@ def load():
     L.usac_gpu_set_neighbors_knn.argtypes = [vp, C.c_int, ip, C.c_int]
     L.usac_gpu_build_neighbors_knn.argtypes = [vp, C.c_int, C.c_int]
     L.usac_gpu_get_neighbors_knn.argtypes = [vp, C.c_int, ip, ip]
+    L.usac_gpu_set_pnapsac_length.argtypes = [vp, C.c_int, C.c_ulonglong]
     L.usac_gpu_set_sprt_pool.argtypes = [vp, C.c_int, ip]
     L.usac_gpu_score.argtypes = [vp, C.c_int, fp, C.c_int, C.c_float, ip, fp]
     L.usac_gpu_errors.argtypes = [vp, C.c_int, fp, fp]

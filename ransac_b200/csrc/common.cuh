@@ -49,7 +49,13 @@ struct ProblemDesc {
     // PROSAC growth function / termination table / SPRT pool offsets (n or n+1 entries each, -1 = absent)
     long long growth_off, term_off, pool_off;
     long long cursor_off;  // NAPSAC per-point use counters (n entries)
+    unsigned long long pn_len;   // Progressive NAPSAC: local samples before the sampler turns global (usac_gpu_set_pnapsac_length); 0 = 20 n
 };
+
+// Progressive NAPSAC (DESIGN.md section 4.8): the hypothesis id at which sampling turns uniform
+__host__ __device__ __forceinline__ unsigned long long pnapsac_length(const ProblemDesc& pd) {
+    return pd.pn_len ? pd.pn_len : 20ull * (unsigned long long)pd.n;
+}
 
 // Evolving state of one robust fit (Ransac::run locals, ransac.cpp:17-56), resident in HBM between rounds.
 struct FitState {

@@ -200,7 +200,10 @@ __global__ void napsac_seed_kernel(const RoundArgs a) {
     const ProblemDesc pd = a.prob[pid];
     const uint64_t hyp = (a.hyp_base_p1 ? (uint64_t)(a.hyp_base_p1 - 1) : (uint64_t)a.state[pid].samples_drawn) + j;
     int p = 0;
-    if (a.neighbors == USAC_NEIGH_KNN) {
+    if (a.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC) {
+        if (hyp >= pnapsac_length(pd)) p = -1;                             // global phase: no centre, nothing counted
+        else philox_unique(a.seed, hyp, 5, pd.n, 1, &p);
+    } else if (a.neighbors == USAC_NEIGH_KNN) {
         philox_unique(a.seed, hyp, 4, pd.n, 1, &p);
     } else {
         // napsac_sampler.hpp:100-128: redraw the seed until its cell holds enough neighbours; a call that finds none in n draws switches
@@ -237,10 +240,42 @@ __global__ void napsac_commit_kernel(const RoundArgs a) {
         const ProblemDesc pd = a.prob[pid];
         const uint64_t hyp = (a.hyp_base_p1 ? (uint64_t)(a.hyp_base_p1 - 1) : (uint64_t)a.state[pid].samples_drawn) + j;
         const bool uniform_by_now = a.neighbors != USAC_NEIGH_KNN && hyp >= (uint64_t)a.cursors[pd.cursor_off + 3 * (size_t)pd.n];
-        if (!uniform_by_now) atomicAdd(&a.cursors[pd.cursor_off + p], (unsigned)(a.m - 1));   // a sample drawn uniformly consumed no neighbours
+        // NAPSAC counts consumed neighbours, Progressive NAPSAC counts uses of the centre; a sample drawn uniformly consumed none
+        const unsigned step = a.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC ? 1u : (unsigned)(a.m - 1);
+        if (!uniform_by_now) atomicAdd(&a.cursors[pd.cursor_off + p], step);
         a.cursors[pd.cursor_off + pd.n + p] = 0u;                     // use count and first user back to zero for the next round
         a.cursors[pd.cursor_off + 2 * (size_t)pd.n + p] = 0u;
     }
+}
+
+// How many samples of this round before sample j share its seed point p (napsac_seed_kernel's use count and first user answer the
+// common cases without a search)
+__device__ __forceinline__ unsigned earlier_uses_in_round(const RoundArgs& a, const ProblemDesc& pd, const int* seeds, int j, int p) {
+    const unsigned uses = a.cursors[pd.cursor_off + pd.n + p];
+    if (uses == 2u)                                                                  // the round draws this seed twice: am I the second one?
+        return ((unsigned)j > (unsigned)a.K - a.cursors[pd.cursor_off + 2 * (size_t)pd.n + p]) ? 1u : 0u;
+    if (uses <= 1u) return 0u;
+    unsigned earlier = 0;                                                            // rarer still: count the earlier uses within this round
+    int i = 0;
+    for (; i + 8 <= j; i += 8) {
+        int v[8];
+#pragma unroll
+        for (int u = 0; u < 8; u++) v[u] = seeds[i + u];
+#pragma unroll
+        for (int u = 0; u < 8; u++) earlier += (v[u] == p);
+    }
+    for (; i < j; i++) earlier += (seeds[i] == p);
+    return earlier;
+}
+
+// Progressive NAPSAC neighbourhood size for the t-th use of a centre (t >= 1): min(k, min{s >= r : C(s, r) >= t}), r = m - 1.
+// PROSAC's growth rule over the centre's own distance-ordered list. C stays below t <= 2^32 until the last step, so the product
+// never leaves 64 bits.
+__device__ __forceinline__ int pnapsac_size(unsigned t, int r, int k) {
+    int s = r;
+    unsigned long long C = 1;                                                        // C(r, r)
+    while (s < k && C < (unsigned long long)t) { C = C * (unsigned long long)(s + 1) / (unsigned long long)(s + 1 - r); s++; }
+    return s;
 }
 
 __global__ void sample_kernel(const RoundArgs a) {
@@ -278,6 +313,25 @@ __global__ void sample_kernel(const RoundArgs a) {
             t_next = t0 + j + 1; n_next = nn;
         }
         if (j == a.K - 1) { st.prosac_t_next = t_next; st.prosac_n_next = n_next; st.prosac_largest_next = max(st.prosac_largest, n_next); }
+    } else if (a.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC) {
+        // DESIGN.md section 4.8: the t-th use of centre p draws from its s(t) nearest neighbours and always takes the s-th one;
+        // t = uses before this round + earlier uses in this round + 1 (the sequential count, whatever the round size)
+        const int* seeds = a.seeds + (size_t)slot * a.K;
+        const int p = seeds[j];
+        if (p < 0) {
+            philox_unique(a.seed, hyp, 0, n, m, s);                                        // global phase: the uniform sampler's sample
+        } else {
+            const unsigned t = a.cursors[pd.cursor_off + p] + earlier_uses_in_round(a, pd, seeds, j, p) + 1u;
+            const int sz = pnapsac_size(t, m - 1, pd.knn);
+            const int* row = a.knn + pd.knn_off + (size_t)pd.knn * p;
+            s[0] = p;
+            s[m - 1] = row[sz - 1];
+            if (m > 2) {
+                int jj[8];
+                philox_unique(a.seed, hyp, 6, sz - 1, m - 2, jj);                          // distinct ranks in [0, s-2]
+                for (int i = 0; i < m - 2; i++) s[1 + i] = row[jj[i]];
+            }
+        }
     } else if (a.sampler == USAC_SAMPLER_NAPSAC) {
         const int* seeds = a.seeds + (size_t)slot * a.K;
         const int p = seeds[j];
@@ -285,23 +339,7 @@ __global__ void sample_kernel(const RoundArgs a) {
         if (p < 0 || uniform_by_now) {
             philox_unique(a.seed, hyp, 0, n, m, s);
         } else {
-            unsigned c = a.cursors[pd.cursor_off + p];
-            const unsigned uses = a.cursors[pd.cursor_off + n + p];
-            if (uses == 2u) {                                                              // the round draws this seed twice: am I the second one?
-                c += ((unsigned)j > (unsigned)a.K - a.cursors[pd.cursor_off + 2 * (size_t)n + p]) ? (unsigned)(m - 1) : 0u;
-            } else if (uses > 2u) {                                                        // rarer still: count the earlier uses within this round
-                unsigned earlier = 0;
-                int i = 0;
-                for (; i + 8 <= j; i += 8) {
-                    int v[8];
-#pragma unroll
-                    for (int u = 0; u < 8; u++) v[u] = seeds[i + u];
-#pragma unroll
-                    for (int u = 0; u < 8; u++) earlier += (v[u] == p);
-                }
-                for (; i < j; i++) earlier += (seeds[i] == p);
-                c += earlier * (unsigned)(m - 1);
-            }
+            const unsigned c = a.cursors[pd.cursor_off + p] + earlier_uses_in_round(a, pd, seeds, j, p) * (unsigned)(m - 1);
             s[0] = p;
             if (a.neighbors == USAC_NEIGH_KNN) {
                 const int* row = a.knn + pd.knn_off + (size_t)pd.knn * p;

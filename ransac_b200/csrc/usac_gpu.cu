@@ -602,6 +602,13 @@ extern "C" int usac_gpu_get_neighbors_knn(usac_gpu_ctx* c, int problem, int* nei
     return USAC_OK;
 }
 
+extern "C" int usac_gpu_set_pnapsac_length(usac_gpu_ctx* c, int problem, unsigned long long local_samples) {
+    if (!c || problem < 0 || problem >= c->P) return fail(c, USAC_ERR_ARG, "set_pnapsac_length: bad arguments");
+    cudaSetDevice(c->device);
+    c->h_prob[problem].pn_len = local_samples;                     // 0: the default, 20 n
+    return push_desc(c);
+}
+
 extern "C" int usac_gpu_set_neighbors_grid(usac_gpu_ctx* c, int problem, int cell_size) {
     if (!c || problem < 0 || problem >= c->P || cell_size <= 0) return fail(c, USAC_ERR_ARG, "set_neighbors_grid: bad arguments");
     if (usac_point_dim(c->est) != 4) return fail(c, USAC_ERR_ARG, "set_neighbors_grid: needs correspondences (nearest_neighbors.cpp:172 reads 4 columns)");
@@ -1058,7 +1065,7 @@ static int setup_sampler_side(usac_gpu_ctx* c, const usac_sampler_cfg& s, bool r
         CUDA_TRY(c, cudaMemcpyAsync(c->d_growth.p, all.data(), sizeof(unsigned) * all.size(), cudaMemcpyHostToDevice, c->stream));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     }
-    if (s.sampler == USAC_SAMPLER_NAPSAC) {
+    if (s.sampler == USAC_SAMPLER_NAPSAC || s.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC) {
         for (int p = 0; p < c->P; p++) {
             const ProblemDesc& d = c->h_prob[p];
             if (s.neighbors == USAC_NEIGH_KNN ? d.knn_off < 0 : d.grid_off < 0) return fail(c, USAC_ERR_STATE, "NAPSAC: neighbourhood of a problem was not set");
@@ -1087,23 +1094,28 @@ static void fill_round_args(usac_gpu_ctx* c, RoundArgs& a, const usac_sampler_cf
     a.rank = 0; a.nranks = 1; a.nchunks = 1;
 }
 
-// Only the samplers that exist: the reference's ProgressiveNapsac never fills its sample (progressive_sampler.hpp:149-172) and
-// Evsac / ProsacNapsac are not wired (init.cpp:23-50) - an unknown enum must not silently become uniform sampling.
+// Only the samplers that exist: Evsac / ProsacNapsac are not wired in the reference (init.cpp:23-50) - an unknown enum must not
+// silently become uniform sampling. Progressive NAPSAC follows DESIGN.md section 4.8 (the reference's progressive_sampler.hpp:149-172
+// never fills its sample).
 static const char* check_sampler_cfg(const usac_sampler_cfg& s) {
-    if (s.sampler != USAC_SAMPLER_UNIFORM && s.sampler != USAC_SAMPLER_NAPSAC && s.sampler != USAC_SAMPLER_PROSAC)
-        return "sampler must be USAC_SAMPLER_UNIFORM, USAC_SAMPLER_NAPSAC or USAC_SAMPLER_PROSAC (Progressive NAPSAC is a stub in the reference and is not built)";
+    if (s.sampler != USAC_SAMPLER_UNIFORM && s.sampler != USAC_SAMPLER_NAPSAC && s.sampler != USAC_SAMPLER_PROSAC &&
+        s.sampler != USAC_SAMPLER_PROGRESSIVE_NAPSAC)
+        return "sampler must be USAC_SAMPLER_UNIFORM, USAC_SAMPLER_PROGRESSIVE_NAPSAC, USAC_SAMPLER_NAPSAC or USAC_SAMPLER_PROSAC";
     if (s.rng != USAC_RNG_PHILOX && s.rng != USAC_RNG_TABLE) return "rng must be USAC_RNG_PHILOX or USAC_RNG_TABLE";
     if (s.sampler == USAC_SAMPLER_NAPSAC && s.neighbors != USAC_NEIGH_KNN && s.neighbors != USAC_NEIGH_GRID)
         return "NAPSAC needs neighbors = USAC_NEIGH_KNN or USAC_NEIGH_GRID";
+    if (s.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC && s.neighbors != USAC_NEIGH_KNN)
+        return "Progressive NAPSAC needs neighbors = USAC_NEIGH_KNN (it grows a distance-ordered neighbourhood; grid cells have no order)";
     return nullptr;
 }
 
 static void launch_sampler(usac_gpu_ctx* c, const RoundArgs& a, int slots) {
     dim3 g((a.K + 127) / 128, slots);
-    if (a.sampler == USAC_SAMPLER_NAPSAC) { napsac_seed_kernel<<<g, 128, 0, c->stream>>>(a); c->last_launches++; }
+    const bool seeded = a.sampler == USAC_SAMPLER_NAPSAC || a.sampler == USAC_SAMPLER_PROGRESSIVE_NAPSAC;
+    if (seeded) { napsac_seed_kernel<<<g, 128, 0, c->stream>>>(a); c->last_launches++; }
     sample_kernel<<<g, 128, 0, c->stream>>>(a);
     c->last_launches++;
-    if (a.sampler == USAC_SAMPLER_NAPSAC) { napsac_commit_kernel<<<g, 128, 0, c->stream>>>(a); c->last_launches++; }
+    if (seeded) { napsac_commit_kernel<<<g, 128, 0, c->stream>>>(a); c->last_launches++; }
 }
 
 static void init_state(FitState& s, const ProblemDesc& d, int est, unsigned max_iterations, uint64_t first_hyp) {

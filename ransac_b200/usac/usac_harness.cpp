@@ -6,10 +6,12 @@
 //   --format evd    header + `x1,y1,x2,y2,FGINN,SNN,detector,descriptor,is_correct` (Reader::readEVDPointsInliers)
 //   --format line2d `width height noise a b c N` + N rows `x y` (dataset/GetImage.h:88-116; the GT line gives the GT inlier count)
 //   --gt-model F    3 x 3 ground-truth model (Reader::getMatrix3x3, the *_model.txt files): GT inliers = points under the threshold
-//   usac_harness <points file> <line2d|homography|fundamental|essential> <uniform|prosac|napsac> <threshold> <confidence> [seed]
+//   usac_harness <points file> <line2d|homography|fundamental|essential> <uniform|prosac|napsac|pnapsac> <threshold> <confidence> [seed]
 //                [--format F] [--gt-model file] [--read-only] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K]
-//                [--all-roots]
+//                [--all-roots] [--pn-length L]
 //                [--report] [--runs N --csv out.csv [--gt-inliers G]]
+// pnapsac (Progressive NAPSAC, DESIGN.md section 4.8) always uses kNN neighbourhoods (--knn, default 5); --pn-length sets its number
+// of local samples (default 20 N).
 // --read-only parses the input, prints `read n=.. dim=.. checksum=.. flagged_inliers=..` and exits (no GPU needed).
 // Prints one `key=value` line per result (model as IEEE bit patterns, inlier ids as a hash) for the parity tests; --report adds the
 // human-readable block of Tests::test (test/test.cpp:38-53); --runs/--csv writes one statistics row in the column layout of
@@ -36,7 +38,9 @@ static void report(const char* tag, Ransac& r, const Model& m) {
     (void)m;
 }
 
-static const char* sampler_name(SAMPLER s) { return s == Uniform ? "uniform" : s == Prosac ? "prosac" : s == Napsac ? "napsac" : "unknown"; }
+static const char* sampler_name(SAMPLER s) {
+    return s == Uniform ? "uniform" : s == Prosac ? "prosac" : s == Napsac ? "napsac" : s == ProgressiveNAPSAC ? "pnapsac" : "unknown";
+}
 static const char* estimator_name(ESTIMATOR e) { return e == Line2d ? "line2d" : e == Homography ? "homography" : e == Fundamental ? "fundamental" : "essential"; }
 
 static void report_block(Ransac& r, const Model& m) {                               // test/test.cpp:38-53
@@ -65,12 +69,12 @@ static Stat stat_of(std::vector<double> v) {
 
 int main(int argc, char** argv) {
     if (argc < 6 || !std::strcmp(argv[1], "--help")) {
-        std::fprintf(stderr, "usage: %s <points.txt> <line2d|homography|fundamental|essential> <uniform|prosac|napsac> <threshold> <confidence> [seed] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K] [--all-roots] [--report] [--runs N --csv out.csv [--gt-inliers G]]\n", argv[0]);
+        std::fprintf(stderr, "usage: %s <points.txt> <line2d|homography|fundamental|essential> <uniform|prosac|napsac|pnapsac> <threshold> <confidence> [seed] [--sequential|--both] [--sprt] [--lo 1|2] [--round K] [--max-iter N] [--knn K] [--all-roots] [--pn-length L] [--report] [--runs N --csv out.csv [--gt-inliers G]]\n", argv[0]);
         return argc < 2 ? 2 : (!std::strcmp(argv[1], "--help") ? 0 : 2);
     }
     const std::string est = argv[2], smp = argv[3];
     const ESTIMATOR e = est == "line2d" ? Line2d : est == "homography" ? Homography : est == "fundamental" ? Fundamental : est == "essential" ? Essential : NullE;
-    const SAMPLER s = smp == "uniform" ? Uniform : smp == "prosac" ? Prosac : smp == "napsac" ? Napsac : NullS;
+    const SAMPLER s = smp == "uniform" ? Uniform : smp == "prosac" ? Prosac : smp == "napsac" ? Napsac : smp == "pnapsac" ? ProgressiveNAPSAC : NullS;
     if (e == NullE || s == NullS) { std::fprintf(stderr, "unknown estimator/sampler\n"); return 2; }
     const int dim = e == Line2d ? 2 : 4;
     std::string format = "pts";
@@ -131,6 +135,7 @@ int main(int argc, char** argv) {
         else if (!std::strcmp(argv[i], "--knn") && i + 1 < argc) knn = std::atoi(argv[++i]);
         else if (!std::strcmp(argv[i], "--sprt")) model.setSprt(true);
         else if (!std::strcmp(argv[i], "--all-roots")) model.setGpuEssentialAllRoots(true);   // essential: every cheirality-valid root
+        else if (!std::strcmp(argv[i], "--pn-length") && i + 1 < argc) model.setGpuPnapsacLocalSamples(std::strtoull(argv[++i], nullptr, 10));
         else if (!std::strcmp(argv[i], "--round") && i + 1 < argc) model.gpu_round_size = std::atoi(argv[++i]);
         else if (!std::strcmp(argv[i], "--max-iter") && i + 1 < argc) model.max_iterations = (unsigned)std::atoi(argv[++i]);
         else if ((!std::strcmp(argv[i], "--format") || !std::strcmp(argv[i], "--gt-model")) && i + 1 < argc) i++;
@@ -139,6 +144,7 @@ int main(int argc, char** argv) {
     }
     model.setCellSize(50);
     if (s == Napsac) model.setNeighborsType(knn > 0 ? Nanoflann : Grid);
+    if (s == ProgressiveNAPSAC) model.setNeighborsType(Nanoflann);
     if (knn > 0) model.setKNearestNeighbors(knn);
     try {
         if (gt_inliers == 0 && flagged_known) gt_inliers = (int)flagged.size();
