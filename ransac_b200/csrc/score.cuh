@@ -20,6 +20,8 @@ __device__ __forceinline__ float fast_rcp(float x) { float r; asm("rcp.approx.ft
 __device__ __forceinline__ float fast_sqrt(float x) { float r; asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 __device__ __forceinline__ float fast_rsqrt(float x) { float r; asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 __device__ __forceinline__ float2 dup(float x) { return make_float2(x, x); }   // folds into the scalar-broadcast operand form of FFMA2
+// max(|a|, |b|), NaN if either is NaN (fmaxf would return the other operand): one FMNMX.NAN with |.| operands on the ALU pipe
+__device__ __forceinline__ float abs_max_nan(float a, float b) { float r; asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(fabsf(a)), "f"(fabsf(b))); return r; }
 
 // ---- mbarrier / bulk-copy helpers (PTX ISA 8.x, sm_90+) ---------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -58,10 +60,6 @@ __device__ __forceinline__ void bulk_copy_g2s(void* dst_smem, const void* src_gm
 //   w   : (fundamental only) 1/den, so that min(t,0)*w = err - thr.
 // The kernel accumulates em = min(t, 0) [* w] (NaN-safe: fminf drops a NaN) and counts its sign bits; finish() turns
 // (sum of em, count) into the reference's error sum of the inliers.
-
-#ifndef USAC_SQ_H_XONLY
-#define USAC_SQ_H_XONLY 0      // homography rejection test of score_sq.cuh on the x coordinate only (see FastModel<HOMOGRAPHY>::reject)
-#endif
 
 template <int EST> struct FastModel;
 
@@ -131,33 +129,19 @@ template <> struct FastModel<USAC_EST_HOMOGRAPHY> {
         if (oy) { t.y = 1.f; s.y = 0.f; }
         w = t;
     }
-    // score_sq.cuh: true = PROVEN outlier (the forward distance alone exceeds 2 thr by more than its guard band)
-    // The point is a PROVEN outlier iff the returned value is > 0 (a NaN proves nothing): (d1 nz)^2 - (2 thr |nz| + k1)^2.
-    __device__ __forceinline__ float2 reject(const float4 A, const float4 B) const {
-#if USAC_SQ_H_XONLY
-        // One coordinate of the forward distance is enough to PROVE an outlier: |x2 - nx/nz| > 2 thr + k1/|nz| implies d1 > 2 thr.
-        // 6 packed instructions instead of 12; what it cannot reject - the points of a vertical strip of half-width ~2 thr around
-        // the projected x, ~1 % of random points instead of ~0.01 % for the disc - goes to the survivor queue, whose drain is exact.
-        // The value is compared with reject_bound() = k1 (the guard band was derived for the sum of both coordinates: it covers one).
-        const float2 X1 = make_float2(A.x, A.y), Y1 = make_float2(A.z, A.w), X2 = make_float2(B.x, B.y);
+    // score_sq.cuh: the point is a PROVEN outlier iff the returned value is > bound (a NaN proves nothing). Max-norm form of the
+    // forward distance: max(|x2 nz - nx|, |y2 nz - ny|) > 2 thr |nz| + k1, 9 packed FMA-pipe instructions per pair (the
+    // maximum and the comparison go to the ALU pipe). It rejects a subset of what the disc of phase1/sure rejects: |ax| > c
+    // implies that the rounded ax^2 + ay^2 exceeds c^2 (DESIGN.md section 4.2), so it is sound with the same band; the square
+    // lets through at most 4/pi of the disc's survivors. max.NaN keeps a NaN in either coordinate a survivor, as the disc did.
+    __device__ __forceinline__ float2 reject(const float4 A, const float4 B, float2& bound) const {
+        const float2 X1 = make_float2(A.x, A.y), Y1 = make_float2(A.z, A.w), X2 = make_float2(B.x, B.y), Y2 = make_float2(B.z, B.w);
         const float2 nz = __ffma2_rn(dup(h31), X1, __ffma2_rn(dup(h32), Y1, dup(h33)));
         const float2 nx = __ffma2_rn(dup(a11), X1, __ffma2_rn(dup(a12), Y1, dup(a13)));   // -(h11 x1 + h12 y1 + h13)
-        const float2 ax = __ffma2_rn(X2, nz, nx);                                           // nz * (x2 - nx/nz)
-        return __ffma2_rn(dup(-T2p), make_float2(fabsf(nz.x), fabsf(nz.y)), make_float2(fabsf(ax.x), fabsf(ax.y)));   // |ax| - 2 thr |nz|
-#else
-        P1 st;
-        phase1(A, B, st);
-        const float2 az = make_float2(fabsf(st.nz.x), fabsf(st.nz.y));
-        const float2 c = __ffma2_rn(dup(T2p), az, dup(k1));
-        return __ffma2_rn(make_float2(-c.x, -c.y), c, st.sa);
-#endif
-    }
-    __device__ __forceinline__ float reject_bound() const {
-#if USAC_SQ_H_XONLY
-        return k1;
-#else
-        return 0.f;
-#endif
+        const float2 ny = __ffma2_rn(dup(a21), X1, __ffma2_rn(dup(a22), Y1, dup(a23)));
+        const float2 ax = __ffma2_rn(X2, nz, nx), ay = __ffma2_rn(Y2, nz, ny);           // nz * (x2 - nx/nz)
+        bound = __ffma2_rn(dup(T2p), make_float2(fabsf(nz.x), fabsf(nz.y)), dup(k1));
+        return make_float2(abs_max_nan(ax.x, ay.x), abs_max_nan(ax.y, ay.y));
     }
     static __device__ __forceinline__ float finish(float sum_em, int cnt, float thr) { return 0.5f * (sum_em + (float)cnt * (2.f * thr)); }
     static __device__ __forceinline__ float strict_to_em(float err, float thr) { return 2.f * err - 2.f * thr; }
@@ -205,8 +189,9 @@ template <> struct FastModel<USAC_EST_FUNDAMENTAL> {
         band = __ffma2_rn(dup(b1), s.den, dup(b0));
     }
     __device__ __forceinline__ float2 weight(const P1& s) const { return make_float2(fast_rcp(s.den.x), fast_rcp(s.den.y)); }
-    // score_sq.cuh: proven outlier iff the returned value is > 0: (n^2 - b0P) - thrP den, 18 packed instructions
-    __device__ __forceinline__ float2 reject(const float4 A, const float4 B) const {
+    // score_sq.cuh: proven outlier iff the returned value is > bound = 0: (n^2 - b0P) - thrP den, 18 packed instructions
+    __device__ __forceinline__ float2 reject(const float4 A, const float4 B, float2& bound) const {
+        bound = make_float2(0.f, 0.f);
         const float2 X1 = make_float2(A.x, A.y), Y1 = make_float2(A.z, A.w), X2 = make_float2(B.x, B.y), Y2 = make_float2(B.z, B.w);
         const float2 a = __ffma2_rn(dup(f11), X1, __ffma2_rn(dup(f12), Y1, dup(f13)));
         const float2 b = __ffma2_rn(dup(f21), X1, __ffma2_rn(dup(f22), Y1, dup(f23)));
@@ -217,7 +202,6 @@ template <> struct FastModel<USAC_EST_FUNDAMENTAL> {
         const float2 den = __ffma2_rn(d, d, __ffma2_rn(c, c, __ffma2_rn(b, b, __fmul2_rn(a, a))));
         return __ffma2_rn(dup(negthrP), den, __ffma2_rn(n, n, dup(-b0P)));
     }
-    __device__ __forceinline__ float reject_bound() const { return 0.f; }
     __device__ __forceinline__ void eval(const float4 A, const float4 B, float2& t, float2& s, float2& w) const {
         P1 st;
         phase1(A, B, st);
@@ -241,7 +225,9 @@ template <> struct FastModel<USAC_EST_ESSENTIAL> {
     // score_sq.cuh: the one-sided test of phase1/sure without the rsqrt. da = |a1| / L with L = |l12|; da alone beyond
     // 2 thr + (ka / L + k0) proves the outlier:  |a1| / L - 2 thr > ka / L + k0  <=>  v := |a1| - ka > (2 thr + k0) L
     // <=>  v |v| > (2 thr + k0)^2 L^2  (the left side keeps the sign of v, the right side is >= 0). 13 packed instructions, no MUFU.
-    __device__ __forceinline__ float2 reject(const float4 A, const float4 B) const {
+    // Proven outlier iff the returned value is > bound = 0.
+    __device__ __forceinline__ float2 reject(const float4 A, const float4 B, float2& bound) const {
+        bound = make_float2(0.f, 0.f);
         const float2 X1 = make_float2(A.x, A.y), Y1 = make_float2(A.z, A.w), X2 = make_float2(B.x, B.y), Y2 = make_float2(B.z, B.w);
         const float2 l1 = __ffma2_rn(dup(e11), X2, __ffma2_rn(dup(e21), Y2, dup(e31)));
         const float2 l2 = __ffma2_rn(dup(e12), X2, __ffma2_rn(dup(e22), Y2, dup(e32)));
@@ -252,7 +238,6 @@ template <> struct FastModel<USAC_EST_ESSENTIAL> {
         const float2 m = __fmul2_rn(dup(C2), a2);
         return __ffma2_rn(v, make_float2(fabsf(v.x), fabsf(v.y)), make_float2(-m.x, -m.y));   // > 0: proven outlier
     }
-    __device__ __forceinline__ float reject_bound() const { return 0.f; }
     // Two phases, as for the homography: err = (da + db)/2 with da = |p1.l|/|l12| (l = E^T p2) and db >= 0, so da alone
     // beyond 2*thr + (its band + the band of the final sum) proves the outlier; phase2 adds the other epipolar distance.
     #ifdef USAC_E_SINGLE_PHASE   /* tuning experiment (tools/): evaluate both halves for every pair */
@@ -315,12 +300,12 @@ template <> struct FastModel<USAC_EST_LINE2D> {
         s = dup(band);
         w = t;
     }
-    __device__ __forceinline__ float2 reject(const float4 A, const float4) const {   // score_sq.cuh: > 0 = proven outlier
+    __device__ __forceinline__ float2 reject(const float4 A, const float4, float2& bound) const {   // score_sq.cuh: > bound = 0: proven outlier
+        bound = make_float2(0.f, 0.f);
         const float2 X = make_float2(A.x, A.y), Y = make_float2(A.z, A.w);
         const float2 v = __ffma2_rn(dup(a), X, __ffma2_rn(dup(b), Y, dup(c)));
         return make_float2(fabsf(v.x) + (negthr - band), fabsf(v.y) + (negthr - band));
     }
-    __device__ __forceinline__ float reject_bound() const { return 0.f; }
     static __device__ __forceinline__ float finish(float sum_em, int cnt, float thr) { return sum_em + (float)cnt * thr; }
     static __device__ __forceinline__ float strict_to_em(float err, float thr) { return err - thr; }
 };

@@ -4,7 +4,7 @@
 // Replaces Quality::getNumberInliers (quality.hpp:60-101) looping the virtual Estimator::GetError.
 //
 // Observation (ncu, profiles/r2_*): for the models a RANSAC round produces, more than 99 % of the (model, point)
-// evaluations are outliers that a cheap one-sided test proves to be outliers (FastModel<EST>::reject: 13 - 19 packed FP32x2
+// evaluations are outliers that a cheap one-sided test proves to be outliers (FastModel<EST>::reject: 9 - 18 packed FP32x2
 // instructions per pair of points, no MUFU, no division), yet in the round-1 kernel one surviving evaluation out of the 64 of
 // a (warp, point pair) sent the whole warp through the second phase (8 MUFU + ~30 more instructions; 45 % of the kernel's
 // time for the homography, and a warp-wide exit from the loop whenever a value fell inside the guard band). Here the hot
@@ -203,25 +203,24 @@ __global__ void __launch_bounds__(USAC_SCORE_THREADS, USAC_SQ_MIN_CTAS) score_sq
                 else { A = tp[2 * j]; B = tp[2 * j + 1]; }
             };
             int j = 0;
-            const float zb = fm.reject_bound();                                     // proven outlier <=> reject(...) > zb
 #pragma unroll 1
             for (; j + USAC_PPI <= np; j += USAC_PPI) {
-                float2 z[USAC_PPI];
+                float2 z[USAC_PPI], zb[USAC_PPI];                                   // proven outlier <=> z > zb
 #pragma unroll
                 for (int q = 0; q < USAC_PPI; q++) {                               // independent instruction streams
                     float4 A, B;
                     load_pair(j + q, A, B);
-                    z[q] = fm.reject(A, B);
+                    z[q] = fm.reject(A, B, zb[q]);
                 }
                 bool lane_any = false;
 #pragma unroll
-                for (int q = 0; q < USAC_PPI; q++) lane_any = lane_any || !(z[q].x > zb) || !(z[q].y > zb);
+                for (int q = 0; q < USAC_PPI; q++) lane_any = lane_any || !(z[q].x > zb[q].x) || !(z[q].y > zb[q].y);
                 // one vote for the whole trip: in most trips every point is a proven outlier for every model of the warp
-                if (!USAC_SQ_TRIPVOTE || ((EST != USAC_EST_HOMOGRAPHY || USAC_SQ_H_XONLY) && USAC_SQ_TRIPVOTE == 2) || __any_sync(0xffffffffu, lane_any && live)) {
+                if (!USAC_SQ_TRIPVOTE || (EST != USAC_EST_HOMOGRAPHY && USAC_SQ_TRIPVOTE == 2) || __any_sync(0xffffffffu, lane_any && live)) {
 #pragma unroll
                     for (int q = 0; q < USAC_PPI; q++) {                           // everything that is not a proven outlier goes to the queue
-                        sq_push(!(z[q].x > zb) && live, qaddr, ebase + 2 * q);
-                        sq_push(!(z[q].y > zb) && live, qaddr, ebase + 2 * q + 1);
+                        sq_push(!(z[q].x > zb[q].x) && live, qaddr, ebase + 2 * q);
+                        sq_push(!(z[q].y > zb[q].y) && live, qaddr, ebase + 2 * q + 1);
                     }
                     if (__any_sync(0xffffffffu, qaddr > q_limit)) drain();           // rare: some lane's queue is nearly full
                 }
@@ -234,9 +233,10 @@ __global__ void __launch_bounds__(USAC_SCORE_THREADS, USAC_SQ_MIN_CTAS) score_sq
                     if (q < rest) {
                         float4 A, B;
                         load_pair(j + q, A, B);
-                        const float2 z = fm.reject(A, B);
-                        sq_push(!(z.x > zb) && live, qaddr, ebase + 2 * q);
-                        sq_push(!(z.y > zb) && live, qaddr, ebase + 2 * q + 1);
+                        float2 zb;
+                        const float2 z = fm.reject(A, B, zb);
+                        sq_push(!(z.x > zb.x) && live, qaddr, ebase + 2 * q);
+                        sq_push(!(z.y > zb.y) && live, qaddr, ebase + 2 * q + 1);
                     }
                 }
                 if (__any_sync(0xffffffffu, qaddr > q_limit)) drain();
