@@ -157,7 +157,9 @@ class GpuContext:
                     sprt=False, round_size=0, neighbors=NEIGH_NONE, sample_table=None, rank=0, nranks=1, lo=0, lo_params=None,
                     max_hypothesis_test_before_sprt=0, essential_roots=E5_ROOTS_FIRST_VALID):
         """One robust fit per uploaded problem; returns a numpy record array laid out as usac_fit_result (no per-problem
-        Python work: this is what a batched caller uses). essential_roots=E5_ROOTS_ALL_VALID (essential only): every
+        Python work: this is what a batched caller uses). lo=1 (InItLORsc) / 2 (InItFLORsc): local optimisation of every new
+        best model, for every estimator (lines refit with the PCA fit); lo_params = (lo_sample_size, lo_inner_iterations,
+        lo_iterative_iterations, lo_threshold_multiplier), 0 = default. essential_roots=E5_ROOTS_ALL_VALID (essential only): every
         cheirality-valid five-point root is a model, so best_model_idx ranges over 0..9."""
         cfg = capi.FitCfg()
         cfg.sampler = capi.SamplerCfg(sampler, rng, seed, neighbors, 0, 0)

@@ -87,7 +87,7 @@ __host__ __device__ __forceinline__ int usac_sample_size(int est) {
     return est == USAC_EST_LINE2D ? 2 : est == USAC_EST_HOMOGRAPHY ? 4 : est == USAC_EST_FUNDAMENTAL ? 7 : 5;
 }
 __host__ __device__ __forceinline__ int usac_models_per_sample(int est) { return est == USAC_EST_FUNDAMENTAL ? 3 : 1; }
-__host__ __device__ __forceinline__ int usac_point_dim(int est) { return est == USAC_EST_LINE2D ? 2 : 4; }
+__host__ __device__ __forceinline__ constexpr int usac_point_dim(int est) { return est == USAC_EST_LINE2D ? 2 : 4; }
 
 // Philox4x32-10 (Salmon et al. SC'11), the counter-based stream of the Philox sampler mode.
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t out[4]) {

@@ -12,6 +12,7 @@
 //  * scoring with the ordered inlier list (cta_score): lanes = all 1024 threads, errors in the reference's arithmetic
 //    (strict_error), error sum = lane sums + fixed tree stride 512 ... 1.
 #pragma once
+#include <type_traits>
 #include "pipeline.cuh"
 #include "refit.cuh"
 #include "score.cuh"
@@ -78,15 +79,25 @@ __device__ __forceinline__ void lo_tree256(T* tree, int count) {
     __syncthreads();
 }
 
+// one point of estimator EST as loaded from the problem's rows: float2 (x, y) for lines, float4 (x1, y1, x2, y2) for two views
+template <int EST>
+using LoPoint = typename std::conditional<usac_point_dim(EST) == 2, float2, float4>::type;
+
 // The points of virtual lane l (ids[l], ids[l + 256], ...) in order, four gathers in flight: f(point) is called once per point.
-template <class F>
+template <int EST, class F>
 __device__ __forceinline__ void lo_lane_points(const float* __restrict__ pts, const int* ids, int n, int l, F f) {
+    using P = LoPoint<EST>;
     for (int k = l; k < n; k += 4 * REFIT_THREADS) {
-        float4 p[4];
+        P p[4];
+        // lines: defined on every path, or ptxas keeps the float2 array in local memory inside this loop (lo_kernel<LINE2D>)
+        if constexpr (usac_point_dim(EST) == 2) {
+#pragma unroll
+            for (int u = 0; u < 4; u++) p[u] = P{0.f, 0.f};
+        }
 #pragma unroll
         for (int u = 0; u < 4; u++) {
             const int i = k + u * REFIT_THREADS;
-            if (i < n) p[u] = reinterpret_cast<const float4*>(pts)[ids[i]];
+            if (i < n) p[u] = reinterpret_cast<const P*>(pts)[ids[i]];
         }
 #pragma unroll
         for (int u = 0; u < 4; u++) if (k + u * REFIT_THREADS < n) f(p[u]);
@@ -121,7 +132,7 @@ __device__ __forceinline__ void lo_aat_group(const float* __restrict__ pts, cons
     double acc[CNT];
 #pragma unroll
     for (int c = 0; c < CNT; c++) acc[c] = 0.0;
-    lo_lane_points(pts, ids, n, l, [&](const float4& p) {
+    lo_lane_points<EST>(pts, ids, n, l, [&](const float4& p) {
         const float x1 = (sf(s1) * sf(p.x) + sf(t1x)).v, y1 = (sf(s1) * sf(p.y) + sf(t1y)).v;
         const float x2 = (sf(s2) * sf(p.z) + sf(t2x)).v, y2 = (sf(s2) * sf(p.w) + sf(t2y)).v;
         float r[2][9];
@@ -142,7 +153,8 @@ __device__ __forceinline__ void lo_aat_group(const float* __restrict__ pts, cons
     for (int c = 0; c < CNT; c++) tree[(G + 4 * c) * REFIT_THREADS + l] = acc[c];
 }
 
-// Estimator::EstimateModelNonMinimalSample on `n` point ids -> sh.model, sh.ok. Same arithmetic as nonminimal_kernel (refit.cuh).
+// Estimator::EstimateModelNonMinimalSample on `n` point ids -> sh.model, sh.ok: the normalised DLT / eight-point path of the two-view
+// estimators; lines are the specialisation below.
 template <int EST>
 __device__ void cta_nonminimal(const float* __restrict__ pts, const int* ids, int n, LoShared& sh) {
     const int t = threadIdx.x;
@@ -156,7 +168,7 @@ __device__ void cta_nonminimal(const float* __restrict__ pts, const int* ids, in
     // ---- normalising transformations: group g sums coordinate g ----
     {
         float a = 0.f;
-        lo_lane_points(pts, ids, n, l, [&](const float4& p) { a = __fadd_rn(a, grp == 0 ? p.x : grp == 1 ? p.y : grp == 2 ? p.z : p.w); });
+        lo_lane_points<EST>(pts, ids, n, l, [&](const float4& p) { a = __fadd_rn(a, grp == 0 ? p.x : grp == 1 ? p.y : grp == 2 ? p.z : p.w); });
         treef[grp * REFIT_THREADS + l] = a;
     }
     lo_tree256<float>(treef, 4);
@@ -166,7 +178,7 @@ __device__ void cta_nonminimal(const float* __restrict__ pts, const int* ids, in
     if (grp < 2) {                                                     // group 0: mean distance in image 1, group 1: in image 2
         float d = 0.f;
         const float mx = grp == 0 ? m[0] : m[2], my = grp == 0 ? m[1] : m[3];
-        lo_lane_points(pts, ids, n, l, [&](const float4& p) {
+        lo_lane_points<EST>(pts, ids, n, l, [&](const float4& p) {
             const sf a = sf(grp == 0 ? p.x : p.z) - sf(mx), b = sf(grp == 0 ? p.y : p.w) - sf(my);
             d = __fadd_rn(d, ssqrt(a * a + b * b).v);
         });
@@ -222,8 +234,34 @@ __device__ void cta_nonminimal(const float* __restrict__ pts, const int* ids, in
     __syncthreads();
 }
 
+// Line2d (line2d_estimator.hpp:59-106): the five sums x, y, xy, xx, yy over the points. Group g accumulates sum g and, group 0, also
+// sum 4 - each sum's addends in its lane's order - then one fixed tree over the five, then the closed form (line_from_sums) on thread 0.
+template <>
+__device__ void cta_nonminimal<USAC_EST_LINE2D>(const float* __restrict__ pts, const int* ids, int n, LoShared& sh) {
+    const int t = threadIdx.x;
+    const int l = t & (REFIT_THREADS - 1), grp = t >> 8;
+    float* treef = reinterpret_cast<float*>(sh.tree);
+    __syncthreads();                                                   // everyone has read the previous call's sh.ok / sh.model
+    if (t == 0) sh.ok = 0;
+    if (n < 2) { __syncthreads(); return; }                            // uniform
+    float a = 0.f, yy = 0.f;
+    lo_lane_points<USAC_EST_LINE2D>(pts, ids, n, l, [&](const float2& p) {
+        a = __fadd_rn(a, grp == 0 ? p.x : grp == 1 ? p.y : grp == 2 ? __fmul_rn(p.x, p.y) : __fmul_rn(p.x, p.x));
+        if (grp == 0) yy = __fadd_rn(yy, __fmul_rn(p.y, p.y));
+    });
+    treef[grp * REFIT_THREADS + l] = a;
+    if (grp == 0) treef[4 * REFIT_THREADS + l] = yy;
+    lo_tree256<float>(treef, 5);
+    if (t == 0) {
+        float r[5];
+        for (int k = 0; k < 5; k++) r[k] = treef[k * REFIT_THREADS];
+        sh.ok = line_from_sums(r, n, sh.model) ? 1 : 0;
+    }
+    __syncthreads();
+}
+
 // Estimator::EstimateModelNonMinimalSample as a kernel of its own (usac_gpu_estimate_nonminimal, the final refit): the CTA-wide
-// form above - one pass for the 45 sums of A'A instead of nonminimal_kernel's 45 (same sums, same order, same bits).
+// form above, for every estimator.
 template <int EST>
 __global__ void __launch_bounds__(LO_THREADS, 1) nonminimal_cta_kernel(const float* __restrict__ pts, const int* __restrict__ ids, int n,
                                                                        float* __restrict__ model_out, int* __restrict__ ok_out) {
@@ -233,7 +271,7 @@ __global__ void __launch_bounds__(LO_THREADS, 1) nonminimal_cta_kernel(const flo
     __syncthreads();
     if (threadIdx.x == 0) {
         *ok_out = sh.ok;
-        if (sh.ok) for (int i = 0; i < 9; i++) model_out[i] = sh.model[i];
+        if (sh.ok) for (int i = 0; i < (EST == USAC_EST_LINE2D ? 3 : 9); i++) model_out[i] = sh.model[i];
     }
 }
 
@@ -254,8 +292,9 @@ __device__ void cta_score(const float* __restrict__ aos, int n, const float* mod
         const int i = start + t;
         bool in = false;
         if (i < n) {
-            const float4 p = reinterpret_cast<const float4*>(aos)[i];
-            const float e = strict_error<EST>(sh.rec, p.x, p.y, p.z, p.w);
+            float e;
+            if constexpr (usac_point_dim(EST) == 2) { const float2 p = reinterpret_cast<const float2*>(aos)[i]; e = strict_error<EST>(sh.rec, p.x, p.y, 0.f, 0.f); }
+            else { const float4 p = reinterpret_cast<const float4*>(aos)[i]; e = strict_error<EST>(sh.rec, p.x, p.y, p.z, p.w); }
             in = e < thr;
             if (in) acc = __fadd_rn(acc, e);
         }

@@ -6,39 +6,15 @@
 //   line2d       line2d_estimator.hpp:59-106 (PCA)
 // with GetNormalizingTransformation (dlt/normalizing_transformation.cpp:7-112).
 //
-// One CTA of 256 threads per call. Every sum over the points is a "lane sum": thread t adds elements t, t+256, ... in order,
-// then the 256 partials are combined by a fixed binary tree (stride 128 ... 1) - the host restatement used by the parity
+// The kernel is the CTA-wide form in lo.cuh (cta_nonminimal, nonminimal_cta_kernel); this file holds its building blocks. Every
+// sum over the points is a "lane sum": virtual lane l (of 256) adds elements l, l+256, ... in order, then the 256 partials are
+// combined by a fixed binary tree (stride 128 ... 1) - the host restatement used by the parity
 // tests adds in exactly this order, so the models are bit-identical. A is formed in float like the reference, A'A (45 unique
 // entries) is accumulated in double, and the null vector is the eigenvector of its smallest eigenvalue (cyclic Jacobi sweeps, at most 12, ended by the first sweep without a rotation) instead of cv::SVD on A. All arithmetic strict (no FMA contraction).
 #pragma once
 #include "strict_math.cuh"
 
 #define REFIT_THREADS 256
-
-__device__ __forceinline__ float refit_tree_f(float v, float* sm) {      // fixed-order block reduction; result in every thread
-    sm[threadIdx.x] = v;
-    __syncthreads();
-#pragma unroll 1
-    for (int s = REFIT_THREADS / 2; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s) sm[threadIdx.x] = __fadd_rn(sm[threadIdx.x], sm[threadIdx.x + s]);
-        __syncthreads();
-    }
-    const float r = sm[0];
-    __syncthreads();
-    return r;
-}
-__device__ __forceinline__ double refit_tree_d(double v, double* sm) {
-    sm[threadIdx.x] = v;
-    __syncthreads();
-#pragma unroll 1
-    for (int s = REFIT_THREADS / 2; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s) sm[threadIdx.x] = __dadd_rn(sm[threadIdx.x], sm[threadIdx.x + s]);
-        __syncthreads();
-    }
-    const double r = sm[0];
-    __syncthreads();
-    return r;
-}
 
 // Eigenvector of the smallest eigenvalue of the symmetric n x n matrix S (n odd, <= 9; S, V in shared memory): at most 12 Jacobi
 // sweeps in the round-robin order, executed by the first warp. Round r rotates the (n-1)/2 disjoint pairs {(r+k) mod n, (r-k) mod n}:
@@ -117,117 +93,24 @@ __device__ void refit_smallest_eigenvector_warp(double* S, int n, double* vec, d
     __syncwarp();
 }
 
-// ok_out: 1 when a model was written. ids: point ids (within the problem), n of them.
-template <int EST>
-__global__ void __launch_bounds__(REFIT_THREADS) nonminimal_kernel(const float* __restrict__ pts, const int* __restrict__ ids, int n,
-                                                                  float* __restrict__ model_out, int* __restrict__ ok_out) {
-    __shared__ double smd[REFIT_THREADS];
-    __shared__ double S[81], V[81], h[9];
-    float* smf = reinterpret_cast<float*>(smd);
-    const int t = threadIdx.x;
-    const float fn = (float)n;
-    if (EST == USAC_EST_LINE2D) {
-        if (n < 2) { if (t == 0) *ok_out = 0; return; }
-        float a[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-        for (int i = t; i < n; i += REFIT_THREADS) {
-            const float2 p = reinterpret_cast<const float2*>(pts)[ids[i]];
-            a[0] = __fadd_rn(a[0], p.x); a[1] = __fadd_rn(a[1], p.y); a[2] = __fadd_rn(a[2], __fmul_rn(p.x, p.y));
-            a[3] = __fadd_rn(a[3], __fmul_rn(p.x, p.x)); a[4] = __fadd_rn(a[4], __fmul_rn(p.y, p.y));
-        }
-        float r[5];
-        for (int k = 0; k < 5; k++) r[k] = refit_tree_f(a[k], smf);
-        if (t == 0) {
-            const sf sx(r[0]), sy(r[1]), sxy(r[2]), sx2(r[3]), sy2(r[4]), N(fn);
-            const sf mx = sx / N, my = sy / N;
-            const sf c00 = sx2 - sf(2.f) * sx * mx + N * mx * mx;
-            const sf c01 = sxy - sx * my - sy * mx + N * mx * my;
-            const sf c11 = sy2 - sf(2.f) * sy * my + N * my * my;
-            const sd p((double)c00.v), q((double)c01.v), rr((double)c11.v);
-            const sd half = sd(0.5) * (p - rr), rad = dsqrt(half * half + q * q), lam = sd(0.5) * (p + rr) - rad;
-            sd vx = q, vy = lam - p;
-            const sd wx = lam - rr, wy = q;
-            if ((wx * wx + wy * wy).v > (vx * vx + vy * vy).v) { vx = wx; vy = wy; }
-            const sd nn = dsqrt(vx * vx + vy * vy);
-            if (!(nn.v > 0.0)) { vx = sd(1.0); vy = sd(0.0); } else { vx = vx / nn; vy = vy / nn; }
-            const sf A((float)vx.v), B((float)vy.v);
-            const float c = (-A * mx - B * my).v;
-            model_out[0] = A.v; model_out[1] = B.v; model_out[2] = c;
-            *ok_out = (isfinite(A.v) && isfinite(B.v) && isfinite(c)) ? 1 : 0;
-        }
-        return;
-    }
-    if (n < 4) { if (t == 0) *ok_out = 0; return; }
-    // ---- normalising transformations ----
-    float m[4];
-    {
-        float a[4] = {0.f, 0.f, 0.f, 0.f};
-        for (int i = t; i < n; i += REFIT_THREADS) {
-            const float4 p = reinterpret_cast<const float4*>(pts)[ids[i]];
-            a[0] = __fadd_rn(a[0], p.x); a[1] = __fadd_rn(a[1], p.y); a[2] = __fadd_rn(a[2], p.z); a[3] = __fadd_rn(a[3], p.w);
-        }
-        for (int k = 0; k < 4; k++) m[k] = __fdiv_rn(refit_tree_f(a[k], smf), fn);
-    }
-    float d1 = 0.f, d2 = 0.f;
-    for (int i = t; i < n; i += REFIT_THREADS) {
-        const float4 p = reinterpret_cast<const float4*>(pts)[ids[i]];
-        const sf a = sf(p.x) - sf(m[0]), b = sf(p.y) - sf(m[1]), c = sf(p.z) - sf(m[2]), d = sf(p.w) - sf(m[3]);
-        d1 = __fadd_rn(d1, ssqrt(a * a + b * b).v);
-        d2 = __fadd_rn(d2, ssqrt(c * c + d * d).v);
-    }
-    d1 = refit_tree_f(d1, smf);
-    d2 = refit_tree_f(d2, smf);
-    const double SQRT2 = 1.41421356237309504880;
-    const float s1 = (float)(sd(SQRT2) / sd((double)__fdiv_rn(d1, fn))).v, s2 = (float)(sd(SQRT2) / sd((double)__fdiv_rn(d2, fn))).v;
-    const float t1x = (-sf(m[0]) * sf(s1)).v, t1y = (-sf(m[1]) * sf(s1)).v, t2x = (-sf(m[2]) * sf(s2)).v, t2y = (-sf(m[3]) * sf(s2)).v;
-    if (!isfinite(s1) || !isfinite(s2)) { if (t == 0) *ok_out = 0; return; }
-    // ---- A'A, one entry at a time (the rows are rebuilt per entry: 45 cheap passes, the same lane order for every entry) ----
-    constexpr int NROWS = (EST == USAC_EST_HOMOGRAPHY) ? 2 : 1;
-    for (int i = 0; i < 9; i++)
-        for (int j = i; j < 9; j++) {
-            double acc = 0.0;
-            for (int k = t; k < n; k += REFIT_THREADS) {
-                const float4 p = reinterpret_cast<const float4*>(pts)[ids[k]];
-                const float x1 = (sf(s1) * sf(p.x) + sf(t1x)).v, y1 = (sf(s1) * sf(p.y) + sf(t1y)).v;
-                const float x2 = (sf(s2) * sf(p.z) + sf(t2x)).v, y2 = (sf(s2) * sf(p.w) + sf(t2y)).v;
-                float r[2][9];
-                if (EST == USAC_EST_HOMOGRAPHY) {
-                    r[0][0] = -x1; r[0][1] = -y1; r[0][2] = -1.f; r[0][3] = 0.f; r[0][4] = 0.f; r[0][5] = 0.f;
-                    r[0][6] = __fmul_rn(x2, x1); r[0][7] = __fmul_rn(x2, y1); r[0][8] = x2;
-                    r[1][0] = 0.f; r[1][1] = 0.f; r[1][2] = 0.f; r[1][3] = -x1; r[1][4] = -y1; r[1][5] = -1.f;
-                    r[1][6] = __fmul_rn(y2, x1); r[1][7] = __fmul_rn(y2, y1); r[1][8] = y2;
-                } else {
-                    r[0][0] = __fmul_rn(x2, x1); r[0][1] = __fmul_rn(x2, y1); r[0][2] = x2; r[0][3] = __fmul_rn(y2, x1); r[0][4] = __fmul_rn(y2, y1);
-                    r[0][5] = y2; r[0][6] = x1; r[0][7] = y1; r[0][8] = 1.f;
-                }
-                double a2 = 0.0;
-                for (int q = 0; q < NROWS; q++) a2 = __dadd_rn(a2, __dmul_rn((double)r[q][i], (double)r[q][j]));
-                acc = __dadd_rn(acc, a2);
-            }
-            const double v = refit_tree_d(acc, smd);
-            if (t == 0) { S[i * 9 + j] = v; S[j * 9 + i] = v; }
-        }
-    __syncthreads();
-    if (t >= 32) return;
-    refit_smallest_eigenvector_warp(S, 9, h, V);
-    if (t != 0) return;
-    sd M[9], R[9];
-    const sd S1((double)s1), T1x((double)t1x), T1y((double)t1y), S2((double)s2), T2x((double)t2x), T2y((double)t2y);
-    for (int i = 0; i < 3; i++) {
-        M[3 * i] = sd(h[3 * i]) * S1; M[3 * i + 1] = sd(h[3 * i + 1]) * S1;
-        M[3 * i + 2] = (sd(h[3 * i]) * T1x + sd(h[3 * i + 1]) * T1y) + sd(h[3 * i + 2]);
-    }
-    bool ok = true;
-    if (EST == USAC_EST_HOMOGRAPHY) {
-        const sd is2 = sd(1.0) / S2, ux = -(T2x * is2), uy = -(T2y * is2);
-        for (int j = 0; j < 3; j++) { R[j] = is2 * M[j] + ux * M[6 + j]; R[3 + j] = is2 * M[3 + j] + uy * M[6 + j]; R[6 + j] = M[6 + j]; }
-        const sd inv = sd(1.0) / R[8];
-        for (int i = 0; i < 9; i++) { const double v = (R[i] * inv).v; if (!dfinite(v)) ok = false; model_out[i] = (float)v; }
-        model_out[8] = 1.f;
-    } else {
-        for (int j = 0; j < 3; j++) { R[j] = S2 * M[j]; R[3 + j] = S2 * M[3 + j]; R[6 + j] = (T2x * M[j] + T2y * M[3 + j]) + M[6 + j]; }
-        const bool scale = fabsf((float)R[8].v) > 1.1920929e-07f;     // FLT_EPSILON
-        const sd inv = scale ? sd(1.0) / R[8] : sd(1.0);
-        for (int i = 0; i < 9; i++) { const double v = (R[i] * inv).v; if (!dfinite(v)) ok = false; model_out[i] = (float)v; }
-    }
-    *ok_out = ok ? 1 : 0;
+// Line2d non-minimal fit (line2d_estimator.hpp:59-106) from the five lane sums r = (x, y, xy, xx, yy) of n points: mean, scatter,
+// the eigenvector of the scatter's smaller eigenvalue (closed form in double) as the normal (A, B), c = -A mx - B my -> model[0..2].
+// Returns whether all three are finite. Every operation is one rounding, in the order of the host restatement the tests use.
+__device__ __forceinline__ bool line_from_sums(const float* r, int n, float* model) {
+    const sf sx(r[0]), sy(r[1]), sxy(r[2]), sx2(r[3]), sy2(r[4]), N((float)n);
+    const sf mx = sx / N, my = sy / N;
+    const sf c00 = sx2 - sf(2.f) * sx * mx + N * mx * mx;
+    const sf c01 = sxy - sx * my - sy * mx + N * mx * my;
+    const sf c11 = sy2 - sf(2.f) * sy * my + N * my * my;
+    const sd p((double)c00.v), q((double)c01.v), rr((double)c11.v);
+    const sd half = sd(0.5) * (p - rr), rad = dsqrt(half * half + q * q), lam = sd(0.5) * (p + rr) - rad;
+    sd vx = q, vy = lam - p;
+    const sd wx = lam - rr, wy = q;
+    if ((wx * wx + wy * wy).v > (vx * vx + vy * vy).v) { vx = wx; vy = wy; }
+    const sd nn = dsqrt(vx * vx + vy * vy);
+    if (!(nn.v > 0.0)) { vx = sd(1.0); vy = sd(0.0); } else { vx = vx / nn; vy = vy / nn; }
+    const sf A((float)vx.v), B((float)vy.v);
+    const float c = (-A * mx - B * my).v;
+    model[0] = A.v; model[1] = B.v; model[2] = c;
+    return isfinite(A.v) && isfinite(B.v) && isfinite(c);
 }

@@ -900,13 +900,14 @@ extern "C" int usac_gpu_get_inliers(usac_gpu_ctx* c, int problem, const float* m
 static void launch_nonminimal(usac_gpu_ctx* c, const float* aos, const int* d_ids, int n, float* d_model, int* d_ok) {
     static bool attr_set = false;
     if (!attr_set) {
+        cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
         cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
         cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
         cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
         attr_set = true;
     }
     switch (c->est) {
-        case USAC_EST_LINE2D: nonminimal_kernel<USAC_EST_LINE2D><<<1, REFIT_THREADS, 0, c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
+        case USAC_EST_LINE2D: nonminimal_cta_kernel<USAC_EST_LINE2D><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
         case USAC_EST_HOMOGRAPHY: nonminimal_cta_kernel<USAC_EST_HOMOGRAPHY><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
         case USAC_EST_FUNDAMENTAL: nonminimal_cta_kernel<USAC_EST_FUNDAMENTAL><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
         default: nonminimal_cta_kernel<USAC_EST_ESSENTIAL><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
@@ -1236,8 +1237,8 @@ static void launch_winner_est(usac_gpu_ctx* c, const RoundArgs& a, int slots) {
 // ------------------------------------------------------------------------------------------------------------------
 // LO-RANSAC: InnerLocalOptimization::GetModelScore + IterativeLocalOptimization (local_optimization/
 // inner_local_optimization.hpp:74-133, iterative_local_optimization.hpp:61-135), kinds InItLORsc (1) and InItFLORsc (2).
-// The control flow runs on the host inside the round replay; every fit / scoring step is a device call
-// (nonminimal_kernel, inliers_sum_kernel). Random subsets: Philox keyed by (seed, call counter) in place of mt19937
+// One LO call is one device loop (lo.cuh: lo_kernel, or the speculative waves lo_pool_kernel / lo_wave_kernel / lo_commit_kernel),
+// called from the host round replay on every new best model. Random subsets: Philox keyed by (seed, call counter) in place of mt19937
 // seeded from random_device (uniform_random_generator.hpp:11-47).
 // ------------------------------------------------------------------------------------------------------------------
 struct LoRunner {
@@ -1275,15 +1276,20 @@ struct LoRunner {
         static bool attr_set = false;
         if (!attr_set) {
             const int smem = (int)sizeof(LoShared);
+            // first use = instantiation order, which steers nvcc's inliner: the line kernels come after the two-view ones, whose code this
+            // keeps as it was before lines had LO
             CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             attr_set = true;
         }
         return USAC_OK;
@@ -1326,6 +1332,7 @@ struct LoRunner {
             wave_calls++;
             int rc;
             switch (c->est) {
+                case USAC_EST_LINE2D: rc = run_waves<USAC_EST_LINE2D>(wv); break;
                 case USAC_EST_HOMOGRAPHY: rc = run_waves<USAC_EST_HOMOGRAPHY>(wv); break;
                 case USAC_EST_FUNDAMENTAL: rc = run_waves<USAC_EST_FUNDAMENTAL>(wv); break;
                 default: rc = run_waves<USAC_EST_ESSENTIAL>(wv); break;
@@ -1333,6 +1340,7 @@ struct LoRunner {
             if (rc) return rc;
         } else {
             switch (c->est) {
+                case USAC_EST_LINE2D: lo_kernel<USAC_EST_LINE2D><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(a); break;
                 case USAC_EST_HOMOGRAPHY: lo_kernel<USAC_EST_HOMOGRAPHY><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(a); break;
                 case USAC_EST_FUNDAMENTAL: lo_kernel<USAC_EST_FUNDAMENTAL><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(a); break;
                 default: lo_kernel<USAC_EST_ESSENTIAL><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(a); break;
@@ -1404,11 +1412,19 @@ extern "C" void usac_prosac_growth_function(unsigned n, unsigned sample_size, un
     memcpy(out, g.data(), sizeof(unsigned) * n);
 }
 
+// LO settings of usac_gpu_fit / usac_gpu_lo_model_score: the kind, and an inlier subset size that lo_subset can draw (at most 16
+// positions) and that over-determines the model (more than the minimal sample). nullptr when they are valid.
+static const char* check_lo_cfg(int est, const usac_fit_cfg* cfg) {
+    if (cfg->lo != 1 && cfg->lo != 2) return "lo must be 1 (InItLORsc) or 2 (InItFLORsc); GC / IRLS are not built";
+    if (cfg->lo_sample_size && (cfg->lo_sample_size < (unsigned)usac_sample_size(est) + 1 || cfg->lo_sample_size > 16))
+        return "lo_sample_size must be 0 or lie in [sample size + 1, 16]";
+    return nullptr;
+}
+
 extern "C" int usac_gpu_lo_model_score(usac_gpu_ctx* c, int problem, const usac_fit_cfg* cfg, uint64_t* call_counter, float* lo_threshold, float* model, int* inliers,
                                        float* score, unsigned* inner_iters, unsigned* iterative_iters) {
     if (!c || !cfg || problem < 0 || problem >= c->P || !call_counter || !model || !inliers || !score) return fail(c, USAC_ERR_ARG, "lo_model_score: bad arguments");
-    if (cfg->lo != 1 && cfg->lo != 2) return fail(c, USAC_ERR_ARG, "lo_model_score: lo must be 1 (InItLORsc) or 2 (InItFLORsc)");
-    if (c->est == USAC_EST_LINE2D) return fail(c, USAC_ERR_ARG, "lo_model_score: local optimisation of line models is not built");
+    if (const char* why = check_lo_cfg(c->est, cfg)) return fail(c, USAC_ERR_ARG, why);
     if (!(cfg->threshold > 0.f)) return fail(c, USAC_ERR_ARG, "lo_model_score: threshold must be positive");
     cudaSetDevice(c->device);
     int rc = push_desc(c);
@@ -1946,13 +1962,10 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
         return fail(c, USAC_ERR_STATE, "fit: nranks > 1 needs usac_gpu_peer_attach, usac_gpu_nccl_init or usac_gpu_set_allgather");
     if (const char* why = check_sampler_cfg(cfg->sampler)) return fail(c, USAC_ERR_ARG, why);
     if (cfg->sampler.rng == USAC_RNG_TABLE && (!cfg->sample_table || cfg->sample_table_rows == 0)) return fail(c, USAC_ERR_ARG, "fit: empty sample table");
-    if (cfg->lo != 0 && cfg->lo != 1 && cfg->lo != 2) return fail(c, USAC_ERR_ARG, "fit: lo must be 0 (none), 1 (InItLORsc) or 2 (InItFLORsc); GC / IRLS are not built");
-    if (cfg->lo && c->est == USAC_EST_LINE2D) return fail(c, USAC_ERR_ARG, "fit: local optimisation of line models is not built");
+    if (cfg->lo) if (const char* why = check_lo_cfg(c->est, cfg)) return fail(c, USAC_ERR_ARG, why);
     if (cfg->essential_roots != USAC_E5_ROOTS_FIRST_VALID && cfg->essential_roots != USAC_E5_ROOTS_ALL_VALID)
         return fail(c, USAC_ERR_ARG, "fit: essential_roots must be USAC_E5_ROOTS_FIRST_VALID or USAC_E5_ROOTS_ALL_VALID");
     if (cfg->essential_roots && c->est != USAC_EST_ESSENTIAL) return fail(c, USAC_ERR_ARG, "fit: essential_roots applies to essential fits only");
-    if (cfg->lo && cfg->lo_sample_size && (cfg->lo_sample_size < (unsigned)usac_sample_size(c->est) + 1 || cfg->lo_sample_size > 16))
-        return fail(c, USAC_ERR_ARG, "fit: lo_sample_size must lie in [sample size + 1, 16]");
     const bool host_replay = cfg->sprt || cfg->lo || cfg->sampler.sampler == USAC_SAMPLER_PROSAC;
     if (host_replay && nranks > 1) return fail(c, USAC_ERR_ARG, "fit: SPRT / PROSAC termination with hypothesis sharding is not supported");
     cudaSetDevice(c->device);

@@ -64,7 +64,7 @@ with tempfile.TemporaryDirectory() as tmp:
         pts = gen.make(cfg, seed_offset=7000 + case, n=n, inlier_ratio=ratio, **({"clustered": True} if sampler == "napsac" else {}))[0]
         n = len(pts)
         sprt = bool(g.random() < 0.5)
-        lo = 0 if cfg == 1 else int(g.choice([0, 0, 1, 2]))
+        lo = int(g.choice([0, 0, 1, 2]))
         path = os.path.join(tmp, "p.txt")
         with open(path, "w") as fh:
             fh.write(f"{n}\n")

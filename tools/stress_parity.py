@@ -43,7 +43,7 @@ for case in range(CASES):
     K = int(g.choice([1, 7, 32, 100, 256, 512]))
     max_it = int(g.choice([50, 300, 1000]))
     sprt = bool(g.random() < 0.5)
-    lo = int(g.choice([0, 0, 1, 2])) if cfg != 1 else 0
+    lo = int(g.choice([0, 0, 1, 2]))
     sampler = str(g.choice(["uniform", "uniform", "prosac", "napsac"])) if cfg != 1 else "uniform"
     kw = dict(threshold=thr, confidence=conf, max_iterations=max_it, seed=seed, round_size=K)
     okw = dict(threshold=thr, confidence=conf, max_iterations=max_it, seed=seed, rng=O.RNG_PHILOX)
