@@ -121,7 +121,9 @@ typedef struct {
     int rank, nranks;
     /* model.hpp:13,25: LocOpt - 0 NullLO, 1 InItLORsc (inner + iterative LO), 2 InItFLORsc (limited samples); runs on every new
      * best model (ransac.cpp:108-110; local_optimization/inner_local_optimization.hpp:74-133, iterative_local_optimization.hpp), for
-     * every estimator: lines refit with the PCA non-minimal fit (line2d_estimator.hpp:59-106) */
+     * every estimator: lines refit with the PCA non-minimal fit (line2d_estimator.hpp:59-106). A batch (P > 1) without PROSAC and
+     * without a sample table runs the pending LO calls of all its problems in one device step; each record equals the problem
+     * fitted alone with the same round size */
     int lo;
     /* model.hpp:26-29 (Model::setLOParametres): 0 = the reference defaults 14 / 20 / 4 / 10. lo_sample_size must be 0 or lie in
      * [m + 1, 16] (m = the minimal sample: 2 lines, 4 homography, 7 fundamental, 5 essential), else USAC_ERR_ARG */

@@ -406,10 +406,9 @@ __device__ int lo_inner_iteration(const LoArgs& a, const ProblemDesc& pd, LoShar
     return 0;
 }
 
+// One LO call by one CTA: the body of lo_kernel and of lo_batch_kernel
 template <int EST>
-__global__ void __launch_bounds__(LO_THREADS, 1) lo_kernel(const LoArgs a) {
-    extern __shared__ __align__(16) unsigned char lo_smem[];
-    LoShared& sh = *reinterpret_cast<LoShared*>(lo_smem);
+__device__ __forceinline__ void lo_call(const LoArgs& a, LoShared& sh) {
     const int t = threadIdx.x;
     const ProblemDesc pd = a.prob[a.problem];
     // every thread follows the same control flow: the decisions depend on values that all threads read from shared / global memory
@@ -444,6 +443,12 @@ __global__ void __launch_bounds__(LO_THREADS, 1) lo_kernel(const LoArgs a) {
         a.io->inliers = best_inl; a.io->score = best_sum; a.io->lo_thr = lo_thr; a.io->calls = calls;
         a.io->inner_done = inner_done; a.io->iterative_done = iterative_done;
     }
+}
+
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_kernel(const LoArgs a) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_call<EST>(a, *reinterpret_cast<LoShared*>(lo_smem));
 }
 
 // ------------------------------------------------------------------------------------------------------------------------------
@@ -484,9 +489,7 @@ struct LoWaveArgs {
 
 // best model -> pool A, avail (quality->getInliers(best_model)); state from the io record
 template <int EST>
-__global__ void __launch_bounds__(LO_THREADS, 1) lo_pool_kernel(const LoWaveArgs w) {
-    extern __shared__ __align__(16) unsigned char lo_smem[];
-    LoShared& sh = *reinterpret_cast<LoShared*>(lo_smem);
+__device__ __forceinline__ void lo_pool(const LoWaveArgs& w, LoShared& sh) {
     const LoArgs& a = w.a;
     const int t = threadIdx.x;
     const ProblemDesc pd = a.prob[a.problem];
@@ -499,6 +502,11 @@ __global__ void __launch_bounds__(LO_THREADS, 1) lo_pool_kernel(const LoWaveArgs
         s.best_inl = a.io->inliers; s.best_sum = a.io->score; s.avail = min(a.io->inliers, sh.cnt);
         s.lo_thr = a.io->lo_thr; s.calls = a.io->calls; s.inner_done = 0; s.iterative_done = 0; s.next_it = 0; s.finished = 0;
     }
+}
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_pool_kernel(const LoWaveArgs w) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_pool<EST>(w, *reinterpret_cast<LoShared*>(lo_smem));
 }
 
 // subset draws an iteration is expected to make (the prediction of the next iteration's call counter)
@@ -537,9 +545,7 @@ __device__ __forceinline__ bool lo_predicted_threshold(const LoArgs& a, float ac
 }
 
 template <int EST>
-__global__ void __launch_bounds__(LO_THREADS, 1) lo_wave_kernel(const LoWaveArgs w) {
-    extern __shared__ __align__(16) unsigned char lo_smem[];
-    LoShared& sh = *reinterpret_cast<LoShared*>(lo_smem);
+__device__ __forceinline__ void lo_wave(const LoWaveArgs& w, LoShared& sh) {
     const LoArgs& a = w.a;
     const ProblemDesc pd = a.prob[a.problem];
     const LoWaveState s = *w.ws;                                     // written by the previous kernel in the stream
@@ -568,9 +574,14 @@ __global__ void __launch_bounds__(LO_THREADS, 1) lo_wave_kernel(const LoWaveArgs
         o.d_inner = d_inner; o.d_iter = d_iter;
     }
 }
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_wave_kernel(const LoWaveArgs w) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_wave<EST>(w, *reinterpret_cast<LoShared*>(lo_smem));
+}
 
 // walk the wave in iteration order (one CTA): accept, apply the first improvement, stop at a misprediction
-__global__ void __launch_bounds__(LO_THREADS) lo_commit_kernel(const LoWaveArgs w) {
+__device__ __forceinline__ void lo_commit(const LoWaveArgs& w) {
     __shared__ int s_copy_from, s_copy_n;
     const LoArgs& a = w.a;
     LoWaveState& s = *w.ws;
@@ -613,3 +624,37 @@ __global__ void __launch_bounds__(LO_THREADS) lo_commit_kernel(const LoWaveArgs 
         a.io->inner_done = s.inner_done; a.io->iterative_done = s.iterative_done;
     }
 }
+__global__ void __launch_bounds__(LO_THREADS) lo_commit_kernel(const LoWaveArgs w) { lo_commit(w); }
+
+// ------------------------------------------------------------------------------------------------------------------------------
+// Batches: the pending LO calls of many problems (one per problem at most) in one launch. A call's record (LoWaveArgs) names its
+// problem, rows, LoIO and its own A / B lists; the waves give each call its own LoWaveState, LoSpec[] and Bwave. Every call runs
+// the code above on its own state, so each result is that of the call run alone, bit for bit.
+// ------------------------------------------------------------------------------------------------------------------------------
+
+// the candidate models of a batch's calls, read where the round left them: io[k].model = models_raw[src[k]] (w floats, 0 beyond)
+__global__ void lo_load_models_kernel(const float* __restrict__ models_raw, const long long* __restrict__ src, int ncalls, int w, LoIO* __restrict__ io) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ncalls * 9) return;
+    const int k = i / 9, e = i % 9;
+    io[k].model[e] = e < w ? models_raw[src[k] * 9 + e] : 0.f;
+}
+
+// one CTA per call (grid.x = calls): the form for steps with many pending calls, where the other calls keep the GPU busy
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_batch_kernel(const LoWaveArgs* __restrict__ calls) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_call<EST>(calls[blockIdx.x].a, *reinterpret_cast<LoShared*>(lo_smem));
+}
+// the speculative waves of several calls: pool and commit one CTA per call (grid.x), waves grid (inner_iters, variants, calls)
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_pool_batch_kernel(const LoWaveArgs* __restrict__ calls) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_pool<EST>(calls[blockIdx.x], *reinterpret_cast<LoShared*>(lo_smem));
+}
+template <int EST>
+__global__ void __launch_bounds__(LO_THREADS, 1) lo_wave_batch_kernel(const LoWaveArgs* __restrict__ calls) {
+    extern __shared__ __align__(16) unsigned char lo_smem[];
+    lo_wave<EST>(calls[blockIdx.z], *reinterpret_cast<LoShared*>(lo_smem));
+}
+__global__ void __launch_bounds__(LO_THREADS) lo_commit_batch_kernel(const LoWaveArgs* __restrict__ calls) { lo_commit(calls[blockIdx.x]); }

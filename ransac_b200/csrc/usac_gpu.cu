@@ -107,6 +107,11 @@ struct usac_gpu_ctx {
     DevBuf<LoSpec> d_lo_spec;
     DevBuf<LoWaveState> d_lo_ws;
     PinnedBuf<LoWaveState> h_lo_ws;
+    DevBuf<LoWaveArgs> d_lo_calls;            // batched LO steps: one record per pending call, its LoIO and the model it starts from
+    PinnedBuf<LoWaveArgs> h_lo_calls;
+    PinnedBuf<LoIO> h_lo_io;
+    DevBuf<long long> d_lo_src;
+    PinnedBuf<long long> h_lo_src;
     DevBuf<unsigned> d_inl_ballots;          // inlier flags of a large problem (launch_inliers)
     DevBuf<int> d_inl_counts;
     PinnedBuf<int> h_rp_nmodels;              // replay path: the round's results on the host
@@ -177,6 +182,7 @@ struct usac_gpu_ctx {
 };
 
 static std::string g_create_error;
+static cudaError_t set_lo_smem_attributes();
 
 static int fail(usac_gpu_ctx* ctx, int code, const char* msg) {
     if (ctx) ctx->err = msg;
@@ -212,6 +218,13 @@ extern "C" int usac_gpu_create(usac_gpu_ctx** out, int device) {
     }
     cudaEventCreate(&c->ev0);
     cudaEventCreate(&c->ev1);
+    // the LO / non-minimal kernels use more than 48 KB of dynamic shared memory: an opt-in of the device's context, set here after
+    // cudaSetDevice so that every context on every device has it
+    if ((e = set_lo_smem_attributes()) != cudaSuccess) {
+        g_create_error = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e);
+        usac_gpu_destroy(c);
+        return USAC_ERR_CUDA;
+    }
     if ((e = c->d_work.ensure(1)) != cudaSuccess || (e = cudaMemset(c->d_work.p, 0, sizeof(unsigned))) != cudaSuccess) {
         g_create_error = cudaGetErrorString(e);
         delete c;
@@ -242,7 +255,7 @@ extern "C" void usac_gpu_destroy(usac_gpu_ctx* c) {
     c->d_pool.release(); c->d_cursors.release(); c->d_growth.release(); c->d_term.release();
     c->d_samples.release(); c->d_nmodels.release(); c->d_offsets.release(); c->d_mvalid.release(); c->d_part_cnt.release();
     c->d_seeds.release(); c->d_table.release(); c->d_models_raw.release(); c->d_recs.release(); c->d_part_sum.release();
-    c->d_scores.release(); c->d_scores_all.release(); c->d_sprt_res.release(); c->d_sprt_carry.release(); c->d_sprt_count.release(); c->d_inl_ballots.release(); c->d_inl_counts.release(); c->d_lo_bwave.release(); c->d_lo_spec.release(); c->d_lo_ws.release(); c->h_lo_ws.release(); c->h_rp_nmodels.release(); c->h_rp_res.release(); c->h_rp_scores.release(); c->h_rp_models.release(); c->h_rp_state.release(); c->d_model_scores.release(); c->d_pool_pts.release(); c->d_grid_keys.release(); c->d_grid_ints.release(); c->d_grid_temp.release(); c->d_knn_cells.release(); c->d_knn_pts.release(); c->d_work.release(); c->d_items.release(); c->d_item_count.release();
+    c->d_scores.release(); c->d_scores_all.release(); c->d_sprt_res.release(); c->d_sprt_carry.release(); c->d_sprt_count.release(); c->d_inl_ballots.release(); c->d_inl_counts.release(); c->d_lo_bwave.release(); c->d_lo_spec.release(); c->d_lo_ws.release(); c->h_lo_ws.release(); c->d_lo_calls.release(); c->h_lo_calls.release(); c->h_lo_io.release(); c->d_lo_src.release(); c->h_lo_src.release(); c->h_rp_nmodels.release(); c->h_rp_res.release(); c->h_rp_scores.release(); c->h_rp_models.release(); c->h_rp_state.release(); c->d_model_scores.release(); c->d_pool_pts.release(); c->d_grid_keys.release(); c->d_grid_ints.release(); c->d_grid_temp.release(); c->d_knn_cells.release(); c->d_knn_pts.release(); c->d_work.release(); c->d_items.release(); c->d_item_count.release();
     c->d_q_models.release(); c->d_q_recs.release(); c->d_q_sum.release(); c->d_q_err.release(); c->d_q_cnt.release(); c->d_q_ids.release(); c->d_q_ids2.release(); c->d_q_ok.release(); c->d_q_model2.release(); c->d_lo_ids_a.release(); c->d_lo_ids_b.release(); c->d_lo_small.release(); c->d_lo_io.release();
     if (c->h_state) cudaFreeHost(c->h_state);
     if (c->h_active) cudaFreeHost(c->h_active);
@@ -897,15 +910,7 @@ extern "C" int usac_gpu_get_inliers(usac_gpu_ctx* c, int problem, const float* m
 // ------------------------------------------------------------------------------------------------------------------
 // Non-minimal estimation and the final refit (ransac.cpp:157-207)
 // ------------------------------------------------------------------------------------------------------------------
-static void launch_nonminimal(usac_gpu_ctx* c, const float* aos, const int* d_ids, int n, float* d_model, int* d_ok) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
-        cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
-        cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
-        cudaFuncSetAttribute(nonminimal_cta_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LoShared));
-        attr_set = true;
-    }
+static int launch_nonminimal(usac_gpu_ctx* c, const float* aos, const int* d_ids, int n, float* d_model, int* d_ok) {
     switch (c->est) {
         case USAC_EST_LINE2D: nonminimal_cta_kernel<USAC_EST_LINE2D><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
         case USAC_EST_HOMOGRAPHY: nonminimal_cta_kernel<USAC_EST_HOMOGRAPHY><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
@@ -913,6 +918,8 @@ static void launch_nonminimal(usac_gpu_ctx* c, const float* aos, const int* d_id
         default: nonminimal_cta_kernel<USAC_EST_ESSENTIAL><<<1, LO_THREADS, sizeof(LoShared), c->stream>>>(aos, d_ids, n, d_model, d_ok); break;
     }
     c->last_launches++;
+    CUDA_TRY(c, cudaPeekAtLastError());                           // a launch that did not start (no shared-memory opt-in, ...)
+    return USAC_OK;
 }
 
 extern "C" int usac_gpu_estimate_nonminimal(usac_gpu_ctx* c, int problem, const int* ids, int count, float* model_out, int* ok_out) {
@@ -926,7 +933,8 @@ extern "C" int usac_gpu_estimate_nonminimal(usac_gpu_ctx* c, int problem, const 
     CUDA_TRY(c, c->d_q_ok.ensure(1));
     CUDA_TRY(c, cudaMemcpyAsync(c->d_q_ids.p, ids, sizeof(int) * count, cudaMemcpyHostToDevice, c->stream));
     c->last_launches = 0;
-    launch_nonminimal(c, c->d_aos.p + (size_t)d.aos_off * dim, c->d_q_ids.p, count, c->d_q_model2.p, c->d_q_ok.p);
+    const int rc = launch_nonminimal(c, c->d_aos.p + (size_t)d.aos_off * dim, c->d_q_ids.p, count, c->d_q_model2.p, c->d_q_ok.p);
+    if (rc) return rc;
     CUDA_TRY(c, cudaMemcpyAsync(model_out, c->d_q_model2.p, sizeof(float) * w, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaMemcpyAsync(ok_out, c->d_q_ok.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
@@ -960,7 +968,8 @@ extern "C" int usac_gpu_refit(usac_gpu_ctx* c, int problem, const float* model_i
     for (int norm = 0; norm < 4; norm++) {
         float m2[9];
         int ok = 0, c2 = 0;
-        launch_nonminimal(c, aos, cur, best, c->d_q_model2.p, c->d_q_ok.p);                // :173
+        rc = launch_nonminimal(c, aos, cur, best, c->d_q_model2.p, c->d_q_ok.p);           // :173
+        if (rc) return rc;
         prepare_models_kernel<<<1, 32, 0, c->stream>>>(c->est, c->d_q_model2.p, 1, w, threshold, c->d_prob.p, problem, c->d_q_recs.p);
         rc = launch_inliers(c, aos, d.n, c->d_q_recs.p, threshold, alt, alt + d.n);        // :180 (count + ids of the refitted model)
         if (rc) return rc;
@@ -1241,6 +1250,40 @@ static void launch_winner_est(usac_gpu_ctx* c, const RoundArgs& a, int slots) {
 // called from the host round replay on every new best model. Random subsets: Philox keyed by (seed, call counter) in place of mt19937
 // seeded from random_device (uniform_random_generator.hpp:11-47).
 // ------------------------------------------------------------------------------------------------------------------
+// dynamic shared memory above 48 KB for the kernels that hold a LoShared (usac_gpu_create: once per context, after cudaSetDevice).
+// First use = instantiation order, which steers nvcc's inliner: the line kernels come after the two-view ones, whose code this
+// keeps as it was before lines had LO, and the batch kernels after the single-call ones.
+static cudaError_t set_lo_smem_attributes() {
+    const int smem = (int)sizeof(LoShared);
+    const void* kernels[] = {
+        (const void*)lo_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_kernel<USAC_EST_LINE2D>,
+        (const void*)lo_pool_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_pool_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_pool_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_pool_kernel<USAC_EST_LINE2D>,
+        (const void*)lo_wave_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_wave_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_wave_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_wave_kernel<USAC_EST_LINE2D>,
+        (const void*)lo_batch_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_batch_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_batch_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_batch_kernel<USAC_EST_LINE2D>,
+        (const void*)lo_pool_batch_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_pool_batch_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_pool_batch_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_pool_batch_kernel<USAC_EST_LINE2D>,
+        (const void*)lo_wave_batch_kernel<USAC_EST_HOMOGRAPHY>, (const void*)lo_wave_batch_kernel<USAC_EST_FUNDAMENTAL>,
+        (const void*)lo_wave_batch_kernel<USAC_EST_ESSENTIAL>, (const void*)lo_wave_batch_kernel<USAC_EST_LINE2D>,
+        (const void*)nonminimal_cta_kernel<USAC_EST_LINE2D>, (const void*)nonminimal_cta_kernel<USAC_EST_HOMOGRAPHY>,
+        (const void*)nonminimal_cta_kernel<USAC_EST_FUNDAMENTAL>, (const void*)nonminimal_cta_kernel<USAC_EST_ESSENTIAL>,
+    };
+    for (const void* k : kernels) {
+        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+static bool lo_seq_env() {                                        // USAC_GPU_LO_SEQ=1: one CTA per LO call, no speculative waves
+    static const bool seq = getenv("USAC_GPU_LO_SEQ") && atoi(getenv("USAC_GPU_LO_SEQ")) != 0;
+    return seq;
+}
+#define LO_WAVE_LIST_BYTES (256u << 20)   // cap on the waves' candidate lists (inner_iters x variants x n ids per call)
+
 struct LoRunner {
     usac_gpu_ctx* c;
     int problem, kind, m, n, w, dim;
@@ -1249,7 +1292,8 @@ struct LoRunner {
     uint64_t seed, calls = 0;
     unsigned inner_done = 0, iterative_done = 0;
 
-    int init(usac_gpu_ctx* ctx, int problem_, const usac_fit_cfg* cfg) {
+    // the parameters and the state that persists across the calls of one fit (no device work)
+    void setup(usac_gpu_ctx* ctx, int problem_, const usac_fit_cfg* cfg) {
         const float threshold = cfg->threshold;
         c = ctx; problem = problem_; kind = cfg->lo; seed = cfg->sampler.seed;
         if (cfg->lo_sample_size) sample_limit = (int)cfg->lo_sample_size;            // Model::setLOParametres, model.hpp:26-29
@@ -1260,37 +1304,41 @@ struct LoRunner {
         n = d.n; m = usac_sample_size(c->est); w = c->est == USAC_EST_LINE2D ? 3 : 9; dim = usac_point_dim(c->est);
         theta = threshold; lo_thr = threshold;
         step = (threshold * (unsigned)mult - threshold) / (unsigned)iter_iters;        // iterative_local_optimization.hpp:43
+    }
+    // the device arguments of one call
+    LoArgs args(LoIO* io, int* A, int* B) const {
+        LoArgs a;
+        a.aos = c->d_aos.p + (size_t)c->h_prob[problem].aos_off * dim; a.prob = c->d_prob.p; a.problem = problem; a.n = n; a.m = m; a.kind = kind;
+        a.sample_limit = sample_limit; a.inner_iters = inner_iters; a.iter_iters = iter_iters; a.mult = mult; a.theta = theta; a.step = step;
+        a.seed = seed; a.io = io; a.A = A; a.B = B;
+        return a;
+    }
+    // the state sent with a call, and the state its result leaves
+    LoIO io_in(int best_inl, float best_sum) const {
+        LoIO io;
+        memset(&io, 0, sizeof(io));
+        io.inliers = best_inl; io.score = best_sum; io.lo_thr = lo_thr; io.calls = calls;
+        return io;
+    }
+    void io_out(const LoIO& io, float* best_model, int& best_inl, float& best_sum) {
+        for (int i = 0; i < w; i++) best_model[i] = io.model[i];
+        best_inl = io.inliers; best_sum = io.score; lo_thr = io.lo_thr; calls = io.calls;
+        inner_done += io.inner_done; iterative_done += io.iterative_done;
+    }
+
+    int init(usac_gpu_ctx* ctx, int problem_, const usac_fit_cfg* cfg) {
+        setup(ctx, problem_, cfg);
         CUDA_TRY(c, c->d_lo_ids_a.ensure((size_t)n));
         CUDA_TRY(c, c->d_lo_ids_b.ensure((size_t)n));
         CUDA_TRY(c, c->d_lo_io.ensure(1));
         // speculative waves (lo.cuh) unless their candidate lists would not fit (inner_iters x variants x n ids) or USAC_GPU_LO_SEQ=1
-        static const bool seq_env = getenv("USAC_GPU_LO_SEQ") && atoi(getenv("USAC_GPU_LO_SEQ")) != 0;
         const size_t lists = (size_t)inner_iters * LO_WAVE_VARIANTS * (size_t)n;
-        waves = !seq_env && lists * sizeof(int) <= (256u << 20);
+        waves = !lo_seq_env() && lists * sizeof(int) <= LO_WAVE_LIST_BYTES;
         if (waves) {
             CUDA_TRY(c, c->d_lo_bwave.ensure(lists));
             CUDA_TRY(c, c->d_lo_spec.ensure((size_t)inner_iters * LO_WAVE_VARIANTS));
             CUDA_TRY(c, c->d_lo_ws.ensure(1));
             CUDA_TRY(c, c->h_lo_ws.ensure(1));
-        }
-        static bool attr_set = false;
-        if (!attr_set) {
-            const int smem = (int)sizeof(LoShared);
-            // first use = instantiation order, which steers nvcc's inliner: the line kernels come after the two-view ones, whose code this
-            // keeps as it was before lines had LO
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_pool_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_HOMOGRAPHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_FUNDAMENTAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_ESSENTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            CUDA_TRY(c, cudaFuncSetAttribute(lo_wave_kernel<USAC_EST_LINE2D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            attr_set = true;
         }
         return USAC_OK;
     }
@@ -1317,15 +1365,10 @@ struct LoRunner {
     // InnerLocalOptimization::GetModelScore: model / score updated in place. One launch (lo.cuh), one synchronisation.
     int get_model_score(float* best_model, int& best_inl, float& best_sum) {
         if (best_inl < 12) return USAC_OK;                                              // inner_local_optimization.hpp:76
-        LoIO io;
-        memset(&io, 0, sizeof(io));
+        LoIO io = io_in(best_inl, best_sum);
         for (int i = 0; i < w; i++) io.model[i] = best_model[i];
-        io.inliers = best_inl; io.score = best_sum; io.lo_thr = lo_thr; io.calls = calls;
         CUDA_TRY(c, cudaMemcpyAsync(c->d_lo_io.p, &io, sizeof(io), cudaMemcpyHostToDevice, c->stream));
-        LoArgs a;
-        a.aos = c->d_aos.p + (size_t)c->h_prob[problem].aos_off * dim; a.prob = c->d_prob.p; a.problem = problem; a.n = n; a.m = m; a.kind = kind;
-        a.sample_limit = sample_limit; a.inner_iters = inner_iters; a.iter_iters = iter_iters; a.mult = mult; a.theta = theta; a.step = step;
-        a.seed = seed; a.io = c->d_lo_io.p; a.A = c->d_lo_ids_a.p; a.B = c->d_lo_ids_b.p;
+        const LoArgs a = args(c->d_lo_io.p, c->d_lo_ids_a.p, c->d_lo_ids_b.p);
         if (waves) {
             LoWaveArgs wv;
             wv.a = a; wv.ws = c->d_lo_ws.p; wv.spec = c->d_lo_spec.p; wv.Bwave = c->d_lo_bwave.p;
@@ -1350,12 +1393,99 @@ struct LoRunner {
         CUDA_TRY(c, cudaMemcpyAsync(&io, c->d_lo_io.p, sizeof(io), cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
         CUDA_TRY(c, cudaGetLastError());
-        for (int i = 0; i < w; i++) best_model[i] = io.model[i];
-        best_inl = io.inliers; best_sum = io.score; lo_thr = io.lo_thr; calls = io.calls;
-        inner_done += io.inner_done; iterative_done += io.iterative_done;
+        io_out(io, best_model, best_inl, best_sum);
         return USAC_OK;
     }
 };
+
+// A batched LO step: the pending calls of several problems of a round (one per problem), each on a model still on the device
+// (models_raw at (slot, q)). With many calls pending, one CTA per call (lo_batch_kernel): the calls keep the GPU busy and the
+// waves' 6 x 20 speculative iterations per call would be work for nothing. With few - a small batch, the tail of a large one -
+// the speculative waves of every call side by side (DESIGN 4.7, "Batches": LO_WAVE_MAX_CALLS from tools/lo_batch_time.py).
+#define LO_WAVE_MAX_CALLS 4
+struct LoCall { int slot, q, inl; float score; };
+
+template <int EST>
+static int lo_batch_launch(usac_gpu_ctx* c, int ncalls, bool waves, int inner_iters, unsigned long long& nwaves) {
+    const size_t smem = sizeof(LoShared);
+    const LoWaveArgs* calls = c->d_lo_calls.p;
+    if (!waves) {
+        lo_batch_kernel<EST><<<ncalls, LO_THREADS, smem, c->stream>>>(calls);
+        c->last_launches++;
+        CUDA_TRY(c, cudaPeekAtLastError());
+        return USAC_OK;
+    }
+    lo_pool_batch_kernel<EST><<<ncalls, LO_THREADS, smem, c->stream>>>(calls);
+    c->last_launches++;
+    for (int guard = 0; guard <= inner_iters; guard++) {
+        lo_wave_batch_kernel<EST><<<dim3(inner_iters, LO_WAVE_VARIANTS, ncalls), LO_THREADS, smem, c->stream>>>(calls);
+        lo_commit_batch_kernel<<<ncalls, LO_THREADS, 0, c->stream>>>(calls);
+        c->last_launches += 2;
+        nwaves++;
+        CUDA_TRY(c, cudaMemcpyAsync(c->h_lo_ws.p, c->d_lo_ws.p, sizeof(LoWaveState) * ncalls, cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+        CUDA_TRY(c, cudaGetLastError());
+        bool finished = true;
+        for (int k = 0; k < ncalls; k++) finished = finished && c->h_lo_ws.p[k].finished;
+        if (finished) return USAC_OK;
+    }
+    return fail(c, USAC_ERR_STATE, "local optimisation: the speculative waves did not finish");
+}
+
+// runs `calls` (slots of `active`) and leaves their results in c->h_lo_io; A / B lists are carved at each problem's point offset
+static int lo_batch_step(usac_gpu_ctx* c, const std::vector<LoRunner>& lo, const std::vector<int>& active, const std::vector<LoCall>& calls,
+                         int KS, unsigned long long& nwaves, int& wave_steps) {
+    const int ncalls = (int)calls.size();
+    const int inner_iters = lo[active[calls[0].slot]].inner_iters, w = c->est == USAC_EST_LINE2D ? 3 : 9;
+    size_t lists = 0;
+    for (const LoCall& k : calls) lists += (size_t)inner_iters * LO_WAVE_VARIANTS * (size_t)c->h_prob[active[k.slot]].n;
+    const bool waves = !lo_seq_env() && ncalls <= LO_WAVE_MAX_CALLS && lists * sizeof(int) <= LO_WAVE_LIST_BYTES;
+    CUDA_TRY(c, c->d_lo_calls.ensure((size_t)ncalls));
+    CUDA_TRY(c, c->h_lo_calls.ensure((size_t)ncalls));
+    CUDA_TRY(c, c->d_lo_io.ensure((size_t)ncalls));
+    CUDA_TRY(c, c->h_lo_io.ensure((size_t)ncalls));
+    CUDA_TRY(c, c->d_lo_src.ensure((size_t)ncalls));
+    CUDA_TRY(c, c->h_lo_src.ensure((size_t)ncalls));
+    if (waves) {
+        CUDA_TRY(c, c->d_lo_bwave.ensure(lists));
+        CUDA_TRY(c, c->d_lo_spec.ensure((size_t)ncalls * inner_iters * LO_WAVE_VARIANTS));
+        CUDA_TRY(c, c->d_lo_ws.ensure((size_t)ncalls));
+        CUDA_TRY(c, c->h_lo_ws.ensure((size_t)ncalls));
+        wave_steps++;
+    }
+    size_t boff = 0;
+    for (int k = 0; k < ncalls; k++) {
+        const LoCall& call = calls[k];
+        const LoRunner& r = lo[active[call.slot]];
+        const long long off = c->h_prob[r.problem].aos_off;
+        c->h_lo_io.p[k] = r.io_in(call.inl, call.score);
+        c->h_lo_src.p[k] = (long long)call.slot * KS + call.q;
+        LoWaveArgs& wa = c->h_lo_calls.p[k];
+        wa.a = r.args(c->d_lo_io.p + k, c->d_lo_ids_a.p + off, c->d_lo_ids_b.p + off);
+        wa.ws = nullptr; wa.spec = nullptr; wa.Bwave = nullptr;
+        if (waves) {
+            wa.ws = c->d_lo_ws.p + k; wa.spec = c->d_lo_spec.p + (size_t)k * inner_iters * LO_WAVE_VARIANTS; wa.Bwave = c->d_lo_bwave.p + boff;
+            boff += (size_t)inner_iters * LO_WAVE_VARIANTS * (size_t)r.n;
+        }
+    }
+    CUDA_TRY(c, cudaMemcpyAsync(c->d_lo_io.p, c->h_lo_io.p, sizeof(LoIO) * ncalls, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(c, cudaMemcpyAsync(c->d_lo_calls.p, c->h_lo_calls.p, sizeof(LoWaveArgs) * ncalls, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(c, cudaMemcpyAsync(c->d_lo_src.p, c->h_lo_src.p, sizeof(long long) * ncalls, cudaMemcpyHostToDevice, c->stream));
+    lo_load_models_kernel<<<(ncalls * 9 + 255) / 256, 256, 0, c->stream>>>(c->d_models_raw.p, c->d_lo_src.p, ncalls, w, c->d_lo_io.p);
+    c->last_launches++;
+    int rc;
+    switch (c->est) {
+        case USAC_EST_LINE2D: rc = lo_batch_launch<USAC_EST_LINE2D>(c, ncalls, waves, inner_iters, nwaves); break;
+        case USAC_EST_HOMOGRAPHY: rc = lo_batch_launch<USAC_EST_HOMOGRAPHY>(c, ncalls, waves, inner_iters, nwaves); break;
+        case USAC_EST_FUNDAMENTAL: rc = lo_batch_launch<USAC_EST_FUNDAMENTAL>(c, ncalls, waves, inner_iters, nwaves); break;
+        default: rc = lo_batch_launch<USAC_EST_ESSENTIAL>(c, ncalls, waves, inner_iters, nwaves); break;
+    }
+    if (rc) return rc;
+    CUDA_TRY(c, cudaMemcpyAsync(c->h_lo_io.p, c->d_lo_io.p, sizeof(LoIO) * ncalls, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    CUDA_TRY(c, cudaGetLastError());
+    return USAC_OK;
+}
 
 // inlier mask of one model over the points in their given (quality-sorted) order: Quality::getInliers -> bytes
 static int fetch_mask(usac_gpu_ctx* c, int problem, const float* model, float thr, std::vector<unsigned char>& mask, std::vector<int>& ids) {
@@ -1508,37 +1638,147 @@ __global__ void gather_models_kernel(const float* __restrict__ models_raw, const
     out[i] = models_raw[((size_t)pk.x * KS + pk.y) * 9 + i % 9];
 }
 
-// SPRT rounds for SEVERAL problems in flight (uniform / NAPSAC sampler, no LO): one set of launches per round for all problems
-// that are still searching, then the host replays every problem's K hypotheses (the same replay as below, problem by problem -
-// it needs libm for the SPRT bound) and the models of the new best hypotheses come back through one gather. Per problem the
-// result is that of the one-problem-at-a-time path (rounds of K, test frozen within a round).
-static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_result* results, int K) {
+// One problem's replay of one round in hypothesis order (ransac.cpp:58-139), shared by fit_host_replay and fit_batch_replay.
+// next() walks the hypotheses from the cursor - evaluation costs, SPRT bookkeeping, `iters` - and stops at the next one whose score
+// beats the best (Score::bigger); the caller runs LO on it (ransac.cpp:108-110) and hands the result to accept(), which stores the
+// best and its termination bound. A batch can so pause a problem at a new best, run the LO calls of many problems in one step and
+// resume. finish() closes the round: one SPRT re-design (the test is frozen within a round), the counters.
+struct RoundReplay {
+    int K, S, m;
+    unsigned n, before_sprt, max_iterations;
+    float log_1_p;
+    const SprtModelResult* res;          // SPRT: per-model results of the round (nullptr without SPRT)
+    const int2* scores;                  // without SPRT: (count, sum bits) per model
+    const int* nmodels;
+    unsigned long long hyp0;
+    unsigned iters_round_start;
+    long long last_improving = -1;
+    unsigned long long rej_inl = 0, rej_pts = 0, evals = 0, useful = 0;
+    bool stopped = false, done = false;  // done: the fit ended inside this round
+    int j = 0, i = 0;                    // cursor: model i of sample j is next
+
+    RoundReplay(const FitState& hs, const usac_fit_cfg* cfg, unsigned n_, int K_, int S_, int m_, const SprtModelResult* res_,
+                const int2* scores_, const int* nmodels_)
+        : K(K_), S(S_), m(m_), n(n_), before_sprt(cfg->max_hypothesis_test_before_sprt ? cfg->max_hypothesis_test_before_sprt : 20u),   // model.hpp:39
+          max_iterations(cfg->max_iterations), log_1_p((float)logf(1 - cfg->confidence)), res(res_), scores(scores_), nmodels(nmodels_),
+          hyp0(hs.samples_drawn), iters_round_start(hs.iters) {}
+
+    bool next(FitState& hs, int& q, int& inl, float& score) {
+        for (; j < K; j++, i = 0) {
+            if (i == 0 && !stopped && !(hs.iters < hs.max_iters)) { stopped = true; done = true; }
+            for (; i < nmodels[j]; i++) {
+                q = j * S + i;
+                unsigned long long cost;
+                if (res) cost = (unsigned long long)res[q].tested_pts + ((!res[q].good && hyp0 + j < before_sprt) ? (unsigned long long)(n - res[q].tested_pts) : 0ull);
+                else cost = n;
+                evals += cost;
+                if (stopped) continue;
+                useful += cost;
+                if (res) {
+                    const SprtModelResult& r = res[q];
+                    if (r.good) { if (r.tested_inl > hs.best_cnt) last_improving = r.tested_inl; }
+                    else { rej_inl += (unsigned long long)r.tested_inl; rej_pts += (unsigned long long)r.tested_pts; }
+                    if (!r.good && hs.iters >= before_sprt) { hs.iters++; continue; }       // ransac.cpp:77-85
+                    inl = r.full_inl; score = (float)inl;                           // sprt.hpp:240-241
+                } else {
+                    inl = scores[q].x; memcpy(&score, &scores[q].y, 4);
+                }
+                if (inl > hs.best_cnt || (inl == hs.best_cnt && score > hs.best_sum)) { i++; return true; }   // Score::bigger
+            }
+            if (!stopped) hs.iters++;
+        }
+        return false;
+    }
+    // the best of hypothesis q after LO; `model` = nullptr leaves hs.best_model to the caller. prosac_bound >= 0: PROSAC's bound
+    void accept(FitState& hs, SprtHost* sprt, int q, int inl, float score, const float* model, int w, long long prosac_bound = -1) {
+        hs.best_cnt = inl; hs.best_sum = score; hs.best_hyp = (long long)(hyp0 + q / S); hs.best_midx = q % S;
+        if (model) for (int k = 0; k < w; k++) hs.best_model[k] = model[k];
+        hs.max_iters = prosac_bound >= 0 ? (unsigned)prosac_bound : standard_termination_value((unsigned)inl, n, m, log_1_p, max_iterations);
+        if (sprt) hs.max_iters = std::min(hs.max_iters, sprt->upper_bound(inl));   // ransac.cpp:129-133
+    }
+    void finish(FitState& hs, SprtHost* sprt) {
+        if (sprt) {
+            const SprtTestH t = sprt->current();
+            double eps = t.epsilon, delta = t.delta;
+            bool redesign = false;
+            if (last_improving >= 0) { eps = (float)last_improving / n; redesign = true; }
+            if (rej_pts > 0) {
+                const float delta_estimated = (float)rej_inl / (unsigned)rej_pts;
+                if (delta_estimated > 0 && std::fabs(t.delta - delta_estimated) / t.delta > 0.05) { delta = delta_estimated; redesign = true; }
+            }
+            if (redesign) sprt->push(eps, delta, (int)iters_round_start);
+            sprt->cursor = (unsigned)(((unsigned long long)sprt->cursor + 32ull * (unsigned long long)K * S) % n);
+            hs.sprt_ntests = (int)sprt->hist.size();
+        }
+        hs.samples_drawn += (unsigned)K;
+        hs.rounds++;
+        hs.evals += evals;
+        hs.useful_evals += useful;
+    }
+};
+
+static void fill_result(const FitState& hs, int w, usac_fit_result& r) {
+    memset(&r, 0, sizeof(r));
+    for (int i = 0; i < w; i++) r.model[i] = hs.best_model[i];
+    r.inliers = hs.best_cnt; r.score = hs.best_sum; r.iterations = hs.iters; r.samples_drawn = hs.samples_drawn;
+    r.best_hyp = hs.best_hyp; r.best_model_idx = hs.best_midx; r.rounds = hs.rounds; r.evals = hs.evals; r.useful_evals = hs.useful_evals;
+}
+
+// SPRT and / or LO rounds for SEVERAL problems in flight (uniform / NAPSAC samplers): one set of launches per round for every
+// problem still searching (the SPRT walks, or the scoring kernel + per-model scores), one copy of the per-model results, then the
+// host replays every problem's K hypotheses (RoundReplay, as fit_host_replay). A problem pauses at a new best that LO works on
+// (>= 12 inliers, inner_local_optimization.hpp:76); the paused problems' calls run as one batched LO step (lo_batch_step) and their
+// replays resume - one sync per round plus one per LO step. The models of new bests that LO did not touch come back through one
+// gather. Rounds stay K (no growth) and without SPRT each problem's points are chunked as in a fit of its own, so every record is
+// that of the problem fitted alone.
+static int fit_batch_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_result* results, int K) {
     const int P = c->P, m = usac_sample_size(c->est), S = fit_models_per_sample(c->est, cfg), w = c->est == USAC_EST_LINE2D ? 3 : 9;
-    const float log_1_p = (float)logf(1 - cfg->confidence);
+    const bool is_sprt = cfg->sprt != 0, is_lo = cfg->lo != 0;
     const int KS = K * S;
-    const unsigned before_sprt = cfg->max_hypothesis_test_before_sprt ? cfg->max_hypothesis_test_before_sprt : 20u;
-    int rc = ensure_round_buffers(c, P, K, 1, 1, S);
+    const int mblocks = (KS + USAC_SCORE_THREADS - 1) / USAC_SCORE_THREADS;
+    // chunk plan of each problem as a fit of its own plans it (the error sums add the chunks' partial sums in order)
+    std::vector<int2> plan(P);
+    int max_chunks = 1;
+    for (int p = 0; p < P; p++) {
+        plan[p] = make_int2(c->h_prob[p].n_pairs, 1);
+        if (!is_sprt) plan_chunks(c, 1, mblocks, c->h_prob[p].n_pairs, &plan[p].x, &plan[p].y);
+        max_chunks = std::max(max_chunks, plan[p].y);
+    }
+    int rc = ensure_round_buffers(c, P, K, max_chunks, 1, S);
     if (rc) return rc;
     CUDA_TRY(c, c->h_rp_nmodels.ensure((size_t)P * K));
-    CUDA_TRY(c, c->h_rp_res.ensure((size_t)P * KS));
+    if (is_sprt) CUDA_TRY(c, c->h_rp_res.ensure((size_t)P * KS));
+    CUDA_TRY(c, c->h_rp_scores.ensure((size_t)P * KS + P));           // per-model scores, then the gather's (slot, q) picks
+    CUDA_TRY(c, c->d_model_scores.ensure((size_t)P * KS + P));        // the same on the device
     CUDA_TRY(c, c->h_rp_models.ensure((size_t)P * 9));
-    CUDA_TRY(c, c->h_rp_scores.ensure((size_t)P));                    // int2 picks (slot, q)
-    CUDA_TRY(c, c->d_model_scores.ensure((size_t)P));                 // the same on the device
     CUDA_TRY(c, c->d_q_models.ensure((size_t)P * 9));
-    std::vector<SprtHost> sprt(P);
+    if (is_lo) {
+        CUDA_TRY(c, c->d_lo_ids_a.ensure((size_t)c->total_points));
+        CUDA_TRY(c, c->d_lo_ids_b.ensure((size_t)c->total_points));
+    }
+    std::vector<SprtHost> sprt(is_sprt ? P : 0);
+    std::vector<LoRunner> lo(is_lo ? P : 0);
     std::vector<int> active(P);
     for (int p = 0; p < P; p++) {
         init_state(c->h_state[p], c->h_prob[p], c->est, cfg->max_iterations, 0);
-        sprt[p].init(c->est, (unsigned)c->h_prob[p].n, (unsigned)m, cfg->max_iterations);
+        if (is_sprt) sprt[p].init(c->est, (unsigned)c->h_prob[p].n, (unsigned)m, cfg->max_iterations);
+        if (is_lo) lo[p].setup(c, p, cfg);
         active[p] = p;
     }
+    static const bool trace = getenv("USAC_GPU_TRACE") != nullptr;
+    int n_rounds = 0, n_lo = 0, n_lo_steps = 0, wave_steps = 0;
+    unsigned long long n_waves = 0;
+    std::vector<RoundReplay> rr;
+    std::vector<int> best_q, run, next;
+    std::vector<LoCall> calls;
     while (!active.empty()) {
+        // slots grouped by chunk plan: one scoring launch per plan
+        if (!is_sprt) std::stable_sort(active.begin(), active.end(), [&](int x, int y) { return plan[x].x < plan[y].x; });
         const int slots = (int)active.size();
         for (int q = 0; q < slots; q++) {
             const int p = active[q];
             FitState& hs = c->h_state[p];
-            const SprtTestH& t = sprt[p].current();
-            hs.sprt_eps = t.epsilon; hs.sprt_delta = t.delta; hs.sprt_A = t.A; hs.sprt_cursor = sprt[p].cursor;
+            if (is_sprt) { const SprtTestH& t = sprt[p].current(); hs.sprt_eps = t.epsilon; hs.sprt_delta = t.delta; hs.sprt_A = t.A; hs.sprt_cursor = sprt[p].cursor; }
             c->h_active[q] = p;
         }
         CUDA_TRY(c, cudaMemcpyAsync(c->d_state.p, c->h_state, sizeof(FitState) * P, cudaMemcpyHostToDevice, c->stream));
@@ -1547,7 +1787,7 @@ static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_res
         fill_round_args(c, a, cfg->sampler, K, S);
         a.thr = cfg->threshold; a.confidence = cfg->confidence; a.max_iterations = cfg->max_iterations;
         a.table_rows = cfg->sample_table_rows; a.nchunks = 1; a.sprt = cfg->sprt; a.pool = c->d_pool.p; a.sprt_res = c->d_sprt_res.p;
-        a.before_sprt = before_sprt;
+        a.before_sprt = cfg->max_hypothesis_test_before_sprt ? cfg->max_hypothesis_test_before_sprt : 20u;
         launch_sampler(c, a, slots);
         switch (c->est) {
             case USAC_EST_LINE2D: launch_solve<USAC_EST_LINE2D>(c, a, slots); break;
@@ -1557,83 +1797,98 @@ static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_res
         }
         prepare_kernel<<<slots, 256, 0, c->stream>>>(a);
         c->last_launches++;
-        switch (c->est) {
-            case USAC_EST_LINE2D: rc = launch_walk<USAC_EST_LINE2D>(c, a, slots); break;
-            case USAC_EST_HOMOGRAPHY: rc = launch_walk<USAC_EST_HOMOGRAPHY>(c, a, slots); break;
-            case USAC_EST_FUNDAMENTAL: rc = launch_walk<USAC_EST_FUNDAMENTAL>(c, a, slots); break;
-            default: rc = launch_walk<USAC_EST_ESSENTIAL>(c, a, slots); break;
+        if (is_sprt) {
+            switch (c->est) {
+                case USAC_EST_LINE2D: rc = launch_walk<USAC_EST_LINE2D>(c, a, slots); break;
+                case USAC_EST_HOMOGRAPHY: rc = launch_walk<USAC_EST_HOMOGRAPHY>(c, a, slots); break;
+                case USAC_EST_FUNDAMENTAL: rc = launch_walk<USAC_EST_FUNDAMENTAL>(c, a, slots); break;
+                default: rc = launch_walk<USAC_EST_ESSENTIAL>(c, a, slots); break;
+            }
+            if (rc) return rc;
+            CUDA_TRY(c, c->h_rp_res.ensure((size_t)P * KS));
+            CUDA_TRY(c, cudaMemcpyAsync(c->h_rp_res.p, c->d_sprt_res.p, sizeof(SprtModelResult) * (size_t)slots * KS, cudaMemcpyDeviceToHost, c->stream));
+        } else {
+            size_t part = 0;                                           // the groups' partial sums follow each other in d_part_*
+            for (int g0 = 0, g1; g0 < slots; g0 = g1) {
+                // one launch per chunk width; the group's chunk grid covers its longest problem (a shorter problem's chunks past its
+                // end hold 0, and adding 0 leaves its sum as it was)
+                int2 pl = plan[active[g0]];
+                for (g1 = g0 + 1; g1 < slots && plan[active[g1]].x == pl.x; g1++) pl.y = std::max(pl.y, plan[active[g1]].y);
+                ScoreArgs sa{};
+                sa.pairs = c->d_pairs.p; sa.aos = c->d_aos.p; sa.prob = c->d_prob.p; sa.active = c->d_active.p + g0;
+                sa.recs = c->d_recs.p + (size_t)g0 * KS * USAC_REC_STRIDE; sa.mvalid = c->d_mvalid.p + g0;
+                sa.M = KS; sa.mstride = KS; sa.chunk_pairs = pl.x; sa.nchunks = pl.y;
+                sa.part_cnt = c->d_part_cnt.p + part; sa.part_sum = c->d_part_sum.p + part;
+                launch_score(c, sa, g1 - g0, mblocks);
+                RoundArgs ga = a;
+                ga.nmodels = a.nmodels + (size_t)g0 * K; ga.offsets = a.offsets + (size_t)g0 * K; ga.nchunks = pl.y;
+                ga.part_cnt = sa.part_cnt; ga.part_sum = sa.part_sum;
+                model_scores_kernel<<<dim3((KS + 127) / 128, g1 - g0), 128, 0, c->stream>>>(ga, c->d_model_scores.p + (size_t)g0 * KS);
+                c->last_launches++;
+                part += (size_t)(g1 - g0) * pl.y * KS;
+            }
+            CUDA_TRY(c, cudaMemcpyAsync(c->h_rp_scores.p, c->d_model_scores.p, sizeof(int2) * (size_t)slots * KS, cudaMemcpyDeviceToHost, c->stream));
         }
-        if (rc) return rc;
-        CUDA_TRY(c, cudaMemcpyAsync(c->h_rp_res.p, c->d_sprt_res.p, sizeof(SprtModelResult) * (size_t)slots * KS, cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(c, cudaMemcpyAsync(c->h_rp_nmodels.p, c->d_nmodels.p, sizeof(int) * (size_t)slots * K, cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));              // the host sync of the round
         CUDA_TRY(c, cudaGetLastError());
+        n_rounds++;
 
+        rr.clear();
+        best_q.assign(slots, -1);                                    // a new best whose model is still on the device (slot, q)
+        run.resize(slots);
+        for (int slot = 0; slot < slots; slot++) {
+            const int p = active[slot];
+            rr.emplace_back(c->h_state[p], cfg, (unsigned)c->h_prob[p].n, K, S, m, is_sprt ? c->h_rp_res.p + (size_t)slot * KS : nullptr,
+                            c->h_rp_scores.p + (size_t)slot * KS, c->h_rp_nmodels.p + (size_t)slot * K);
+            run[slot] = slot;
+        }
+        while (!run.empty()) {                                       // replay until every problem reaches the end of its round
+            calls.clear();
+            for (int slot : run) {
+                const int p = active[slot];
+                FitState& hs = c->h_state[p];
+                int q, inl;
+                float score;
+                while (rr[slot].next(hs, q, inl, score)) {
+                    if (is_lo && inl >= 12) { calls.push_back({slot, q, inl, score}); break; }   // pause: LO works on this one
+                    rr[slot].accept(hs, is_sprt ? &sprt[p] : nullptr, q, inl, score, nullptr, w);
+                    best_q[slot] = q;
+                }
+            }
+            if (calls.empty()) break;
+            rc = lo_batch_step(c, lo, active, calls, KS, n_waves, wave_steps);
+            if (rc) return rc;
+            n_lo += (int)calls.size(); n_lo_steps++;
+            run.clear();
+            for (size_t k = 0; k < calls.size(); k++) {
+                const LoCall& call = calls[k];
+                const int p = active[call.slot];
+                float model[9] = {0};
+                int inl = call.inl;
+                float score = call.score;
+                lo[p].io_out(c->h_lo_io.p[k], model, inl, score);
+                rr[call.slot].accept(c->h_state[p], is_sprt ? &sprt[p] : nullptr, call.q, inl, score, model, w);
+                best_q[call.slot] = -1;
+                run.push_back(call.slot);
+            }
+        }
         int npicks = 0;
-        int2* picks = c->h_rp_scores.p;
+        int2* picks = c->h_rp_scores.p + (size_t)P * KS;
         std::vector<int> pick_problem;
-        std::vector<int> next;
+        next.clear();
         for (int slot = 0; slot < slots; slot++) {
             const int p = active[slot];
             FitState& hs = c->h_state[p];
-            SprtHost& sp = sprt[p];
-            const unsigned n = (unsigned)c->h_prob[p].n;
-            const SprtModelResult* h_res = c->h_rp_res.p + (size_t)slot * KS;
-            const int* h_nmodels = c->h_rp_nmodels.p + (size_t)slot * K;
-            // ---- replay the round in hypothesis order (ransac.cpp:58-139), as fit_host_replay does ----
-            const unsigned long long hyp0 = hs.samples_drawn;
-            const unsigned iters_round_start = hs.iters;
-            long long last_improving = -1;
-            unsigned long long rej_inl = 0, rej_pts = 0, evals = 0, useful = 0;
-            bool stopped = false, done = false;
-            int best_q = -1;
-            for (int j = 0; j < K; j++) {
-                if (!stopped && !(hs.iters < hs.max_iters)) { stopped = true; done = true; }
-                for (int i = 0; i < h_nmodels[j]; i++) {
-                    const int q = j * S + i;
-                    const SprtModelResult& r = h_res[q];
-                    const unsigned long long cost = (unsigned long long)r.tested_pts + ((!r.good && hyp0 + j < before_sprt) ? (unsigned long long)(n - r.tested_pts) : 0ull);
-                    evals += cost;
-                    if (stopped) continue;
-                    useful += cost;
-                    if (r.good) { if (r.tested_inl > hs.best_cnt) last_improving = r.tested_inl; }
-                    else { rej_inl += (unsigned long long)r.tested_inl; rej_pts += (unsigned long long)r.tested_pts; }
-                    if (!r.good && hs.iters >= before_sprt) { hs.iters++; continue; }       // ransac.cpp:77-85
-                    const int inl = r.full_inl;
-                    const float score = (float)inl;                                          // sprt.hpp:240-241
-                    if (inl > hs.best_cnt || (inl == hs.best_cnt && score > hs.best_sum)) {   // Score::bigger
-                        hs.best_cnt = inl; hs.best_sum = score; hs.best_hyp = (long long)(hyp0 + j); hs.best_midx = i;
-                        best_q = q;
-                        hs.max_iters = standard_termination_value((unsigned)inl, n, m, log_1_p, cfg->max_iterations);
-                        hs.max_iters = std::min(hs.max_iters, sp.upper_bound(inl));           // ransac.cpp:129-133
-                    }
-                }
-                if (!stopped) hs.iters++;
-            }
-            {                                                        // one re-design per round (state is frozen within a round)
-                const SprtTestH t = sp.current();
-                double eps = t.epsilon, delta = t.delta;
-                bool redesign = false;
-                if (last_improving >= 0) { eps = (float)last_improving / n; redesign = true; }
-                if (rej_pts > 0) {
-                    const float delta_estimated = (float)rej_inl / (unsigned)rej_pts;
-                    if (delta_estimated > 0 && std::fabs(t.delta - delta_estimated) / t.delta > 0.05) { delta = delta_estimated; redesign = true; }
-                }
-                if (redesign) sp.push(eps, delta, (int)iters_round_start);
-                sp.cursor = (unsigned)(((unsigned long long)sp.cursor + 32ull * (unsigned long long)KS) % n);
-                hs.sprt_ntests = (int)sp.hist.size();
-            }
-            hs.samples_drawn += (unsigned)K;
-            hs.rounds++;
-            hs.evals += evals;
-            hs.useful_evals += useful;
-            if (best_q >= 0) { picks[npicks] = make_int2(slot, best_q); pick_problem.push_back(p); npicks++; }
-            if (!done && hs.iters < hs.max_iters) next.push_back(p);
+            rr[slot].finish(hs, is_sprt ? &sprt[p] : nullptr);
+            if (best_q[slot] >= 0) { picks[npicks] = make_int2(slot, best_q[slot]); pick_problem.push_back(p); npicks++; }
+            if (!rr[slot].done && hs.iters < hs.max_iters) next.push_back(p);
             else hs.done = 1;
         }
-        if (npicks) {                                                // the models of this round's new best hypotheses, one gather
-            CUDA_TRY(c, cudaMemcpyAsync(c->d_model_scores.p, picks, sizeof(int2) * npicks, cudaMemcpyHostToDevice, c->stream));
-            gather_models_kernel<<<(npicks * 9 + 255) / 256, 256, 0, c->stream>>>(c->d_models_raw.p, c->d_model_scores.p, npicks, KS, c->d_q_models.p);
+        if (npicks) {                                                // the models of this round's new bests that LO did not touch, one gather
+            int2* d_picks = c->d_model_scores.p + (size_t)P * KS;
+            CUDA_TRY(c, cudaMemcpyAsync(d_picks, picks, sizeof(int2) * npicks, cudaMemcpyHostToDevice, c->stream));
+            gather_models_kernel<<<(npicks * 9 + 255) / 256, 256, 0, c->stream>>>(c->d_models_raw.p, d_picks, npicks, KS, c->d_q_models.p);
             c->last_launches++;
             CUDA_TRY(c, cudaMemcpyAsync(c->h_rp_models.p, c->d_q_models.p, sizeof(float) * 9 * npicks, cudaMemcpyDeviceToHost, c->stream));
             CUDA_TRY(c, cudaStreamSynchronize(c->stream));
@@ -1648,19 +1903,19 @@ static int fit_sprt_batch(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_res
     for (int p = 0; p < P; p++) {
         const FitState& hs = c->h_state[p];
         usac_fit_result& r = results[p];
-        memset(&r, 0, sizeof(r));
-        for (int i = 0; i < w; i++) r.model[i] = hs.best_model[i];
-        r.inliers = hs.best_cnt; r.score = hs.best_sum; r.iterations = hs.iters; r.samples_drawn = hs.samples_drawn;
-        r.best_hyp = hs.best_hyp; r.best_model_idx = hs.best_midx; r.rounds = hs.rounds; r.evals = hs.evals; r.useful_evals = hs.useful_evals;
-        r.msac = nanf("");
+        fill_result(hs, w, r);
+        if (is_lo) { r.lo_inner_iters = lo[p].inner_done; r.lo_iterative_iters = lo[p].iterative_done; }
+        r.msac = is_sprt ? nanf("") : usac_msac_cost(c->h_prob[p].n, r.inliers, r.score, cfg->threshold);
     }
+    if (trace)
+        fprintf(stderr, "usac_gpu_fit[batch replay] P=%d K=%d rounds=%d: LO %d calls in %d steps (%d with waves, %llu waves)\n",
+                P, K, n_rounds, n_lo, n_lo_steps, wave_steps, n_waves);
     return USAC_OK;
 }
 
 static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_result* results, int K) {
     const int P = c->P, m = usac_sample_size(c->est), S = fit_models_per_sample(c->est, cfg), w = c->est == USAC_EST_LINE2D ? 3 : 9;
     const bool is_prosac = cfg->sampler.sampler == USAC_SAMPLER_PROSAC, is_sprt = cfg->sprt != 0;
-    const float log_1_p = (float)logf(1 - cfg->confidence);
     const int KS = K * S;
     const unsigned before_sprt = cfg->max_hypothesis_test_before_sprt ? cfg->max_hypothesis_test_before_sprt : 20u;   // model.hpp:39
     std::vector<int> ids;
@@ -1829,86 +2084,39 @@ static int fit_host_replay(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_re
             double t_lo_round = 0, t_mask_round = 0;
 
             // ---- replay the round in hypothesis order (ransac.cpp:58-139) ----
-            const unsigned long long hyp0 = hs.samples_drawn;
-            const unsigned iters_round_start = hs.iters;
-            long long last_improving = -1;
-            unsigned long long rej_inl = 0, rej_pts = 0, evals = 0, useful = 0;
-            bool stopped = false;
-            for (int j = 0; j < K; j++) {
-                if (!stopped && !(hs.iters < hs.max_iters)) { stopped = true; done = true; }
-                for (int i = 0; i < h_nmodels[j]; i++) {
-                    const int q = j * S + i;
-                    unsigned long long cost;
-                    if (is_sprt) cost = (unsigned long long)h_res[q].tested_pts + ((!h_res[q].good && hyp0 + j < before_sprt) ? (unsigned long long)(n - h_res[q].tested_pts) : 0ull);
-                    else cost = n;
-                    evals += cost;
-                    if (stopped) continue;
-                    useful += cost;
-                    int inl;
-                    float score;
-                    if (is_sprt) {
-                        const SprtModelResult& r = h_res[q];
-                        if (r.good) { if (r.tested_inl > hs.best_cnt) last_improving = r.tested_inl; }
-                        else { rej_inl += (unsigned long long)r.tested_inl; rej_pts += (unsigned long long)r.tested_pts; }
-                        if (!r.good && hs.iters >= before_sprt) { hs.iters++; continue; }       // ransac.cpp:77-85
-                        inl = r.full_inl; score = (float)inl;                           // sprt.hpp:240-241
-                    } else {
-                        inl = h_scores[q].x; memcpy(&score, &h_scores[q].y, 4);
-                    }
-                    if (inl > hs.best_cnt || (inl == hs.best_cnt && score > hs.best_sum)) {   // Score::bigger
-                        float cand[9] = {0};
-                        for (int k = 0; k < w; k++) cand[k] = h_models[(size_t)q * 9 + k];
-                        if (cfg->lo) {                                                   // ransac.cpp:108-110
-                            const auto t0 = now();
-                            rc = lo.get_model_score(cand, inl, score);
-                            if (rc) return rc;
-                            t_lo_round += us(t0, now()); n_lo++;
-                        }
-                        hs.best_cnt = inl; hs.best_sum = score; hs.best_hyp = (long long)(hyp0 + j); hs.best_midx = i;
-                        for (int k = 0; k < w; k++) hs.best_model[k] = cand[k];
-                        if (is_prosac) {                                                 // ransac.cpp:123-125
-                            const auto t0 = now();
-                            rc = fetch_mask(c, p, hs.best_model, cfg->threshold, mask, ids);
-                            if (rc) return rc;
-                            hs.max_iters = pterm.update(hs.iters, mask, dev_state.prosac_largest_next);
-                            t_mask_round += us(t0, now()); n_mask++;
-                        } else {
-                            hs.max_iters = standard_termination_value((unsigned)inl, n, m, log_1_p, cfg->max_iterations);
-                        }
-                        if (is_sprt) hs.max_iters = std::min(hs.max_iters, sprt.upper_bound(inl));   // ransac.cpp:129-133
-                    }
+            RoundReplay rr(hs, cfg, n, K, S, m, is_sprt ? h_res : nullptr, h_scores, h_nmodels);
+            int q, inl;
+            float score;
+            while (rr.next(hs, q, inl, score)) {
+                float cand[9] = {0};
+                for (int k = 0; k < w; k++) cand[k] = h_models[(size_t)q * 9 + k];
+                if (cfg->lo) {                                                   // ransac.cpp:108-110
+                    const auto t0 = now();
+                    rc = lo.get_model_score(cand, inl, score);
+                    if (rc) return rc;
+                    t_lo_round += us(t0, now()); n_lo++;
                 }
-                if (!stopped) hs.iters++;
-            }
-            if (is_sprt) {                                       // one re-design per round (state is frozen within a round)
-                const SprtTestH t = sprt.current();
-                double eps = t.epsilon, delta = t.delta;
-                bool redesign = false;
-                if (last_improving >= 0) { eps = (float)last_improving / n; redesign = true; }
-                if (rej_pts > 0) {
-                    const float delta_estimated = (float)rej_inl / (unsigned)rej_pts;
-                    if (delta_estimated > 0 && std::fabs(t.delta - delta_estimated) / t.delta > 0.05) { delta = delta_estimated; redesign = true; }
+                long long prosac_bound = -1;
+                if (is_prosac) {                                                 // ransac.cpp:123-125
+                    const auto t0 = now();
+                    rc = fetch_mask(c, p, cand, cfg->threshold, mask, ids);
+                    if (rc) return rc;
+                    prosac_bound = pterm.update(hs.iters, mask, dev_state.prosac_largest_next);
+                    t_mask_round += us(t0, now()); n_mask++;
                 }
-                if (redesign) sprt.push(eps, delta, (int)iters_round_start);
-                sprt.cursor = (unsigned)(((unsigned long long)sprt.cursor + 32ull * (unsigned long long)KS) % n);
-                hs.sprt_ntests = (int)sprt.hist.size();
+                rr.accept(hs, is_sprt ? &sprt : nullptr, q, inl, score, cand, w, prosac_bound);
             }
+            done = rr.done;
             hs.prosac_t = dev_state.prosac_t_next; hs.prosac_n = dev_state.prosac_n_next; hs.prosac_largest = dev_state.prosac_largest_next;
             hs.prosac_t_next = hs.prosac_t; hs.prosac_n_next = hs.prosac_n; hs.prosac_largest_next = hs.prosac_largest;
-            hs.samples_drawn += (unsigned)K;
-            hs.rounds++;
-            hs.evals += evals;
-            hs.useful_evals += useful;
+            rr.finish(hs, is_sprt ? &sprt : nullptr);
             t_lo += t_lo_round; t_mask += t_mask_round;
             t_replay += us(t_r2, now()) - t_lo_round - t_mask_round;
         }
         hs.done = 1;
         if (overlap && prelaunched > (block_round - 1) / G) CUDA_TRY(c, cudaStreamSynchronize(c->stream2));   // solved ahead and never used (rare: see likely_more): its buffers are free again
         usac_fit_result& r = results[p];
-        memset(&r, 0, sizeof(r));
-        for (int i = 0; i < w; i++) r.model[i] = hs.best_model[i];
-        r.inliers = hs.best_cnt; r.score = hs.best_sum; r.iterations = hs.iters; r.samples_drawn = hs.samples_drawn;
-        r.best_hyp = hs.best_hyp; r.best_model_idx = hs.best_midx; r.rounds = hs.rounds; r.evals = hs.evals; r.useful_evals = hs.useful_evals;
+        fill_result(hs, w, r);
         if (cfg->lo) { r.lo_inner_iters = lo.inner_done; r.lo_iterative_iters = lo.iterative_done; n_waves += lo.wave_count; }
         r.msac = is_sprt ? nanf("") : usac_msac_cost(pd.n, r.inliers, r.score, cfg->threshold);
     }
@@ -2037,9 +2245,11 @@ extern "C" int usac_gpu_fit(usac_gpu_ctx* c, const usac_fit_cfg* cfg, usac_fit_r
     if (host_replay) {
         c->score_events_used = 0; c->last_launches = 0; c->last_score_launches = 0;
         cudaEventRecord(c->ev0, c->stream);
-        static const bool batch_off = getenv("USAC_GPU_SPRT_BATCH") && atoi(getenv("USAC_GPU_SPRT_BATCH")) == 0;   // A/B knob
-        const bool batch = !batch_off && c->P > 1 && cfg->sprt && !cfg->lo && cfg->sampler.sampler != USAC_SAMPLER_PROSAC && cfg->sampler.rng != USAC_RNG_TABLE;
-        rc = batch ? fit_sprt_batch(c, cfg, results, K) : fit_host_replay(c, cfg, results, K);
+        // USAC_GPU_SPRT_BATCH=0 (A/B knob): SPRT-only batches one problem at a time
+        static const bool batch_off = getenv("USAC_GPU_SPRT_BATCH") && atoi(getenv("USAC_GPU_SPRT_BATCH")) == 0;
+        const bool batch = c->P > 1 && (cfg->lo || (cfg->sprt && !batch_off)) && cfg->sampler.sampler != USAC_SAMPLER_PROSAC &&
+                           cfg->sampler.rng != USAC_RNG_TABLE;
+        rc = batch ? fit_batch_replay(c, cfg, results, K) : fit_host_replay(c, cfg, results, K);
         cudaEventRecord(c->ev1, c->stream);
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
         collect_timing(c);
